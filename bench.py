@@ -10,6 +10,7 @@ top-k, and the local lists are merged after one NCCL allgather.
 
   python bench.py --gpus 1 --steps 5 --warmup 3                 # ours
   python bench.py --impl reference --gpus 1 --steps 2 --warmup 1 # the restated reference on the host cores
+  python bench.py --steps 5 --warmup 3 --dump-outputs OUT       # + the last timed step's answers as OUT/*.npy
 
 The oracle (oracle/) is used here only as the checker (sample parity) and as the measured CPU baseline.
 """
@@ -47,8 +48,10 @@ def metric_object(z, name):
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 5; preset 4: enough to hash 100M rows)")
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (ordinals, distances, counts) as DIR/<name>.npy")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", type=int, default=1_000_000, help="rows per GPU")
     ap.add_argument("--dim", type=int, default=768)
@@ -85,7 +88,8 @@ def parse():
     if a.preset == 4:
         a.workload, a.dim, a.rows, a.hash_rows, a.scaling = "hash", 768, 1_000_000, 2_500_000, "strong"
         a.total_hash_rows = 100_000_000
-        a.steps = max(1, a.total_hash_rows // (a.gpus * a.hash_rows))
+        if a.steps is None:
+            a.steps = max(1, a.total_hash_rows // (a.gpus * a.hash_rows))
     elif a.preset == 6:
         a.metric, a.dim, a.topk, a.trees = "l2", 768, 10, 3
         a.rows, a.queries, a.scaling = 100_000_000 // a.gpus, max(1, 10_000 // a.gpus), "strong"
@@ -95,6 +99,12 @@ def parse():
     elif a.preset == 5:
         a.metric, a.dim, a.topk, a.delete_frac = "l2sq", 384, 100, 0.1
         a.rows, a.queries, a.scaling = 100_000_000 // a.gpus, max(1, 100_000 // a.gpus), "strong"
+    if a.steps is None:
+        a.steps = 5
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and (a.impl != "ours" or a.workload != "query"):
+        ap.error("--dump-outputs writes the results of the query workload of --impl ours")
     return a
 
 
@@ -110,6 +120,29 @@ def seeded_deletes(total_rows, frac, seed):
         h ^= h >> np.uint64(32)
         out.append(o[(h & np.uint64(0xFFFFFFFF)) < np.uint64(thr)])
     return np.concatenate(out) if out else np.zeros(0, np.uint64)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, metric, ords, bits, counts):
+    """The answers of one query batch as float64 .npy files, exact (ordinals < 2^53; distances are f64 / f32 values or
+    integer counts), so that two builds can be compared value for value.  Slots past a query's count hold ordinal -1 and
+    distance +inf.  A batch whose answers exceed DUMP_BYTES is written for a fixed, seeded sample of its queries;
+    query_rows.npy says which rows of the batch were kept."""
+    nq, k = ords.shape
+    rows = np.arange(nq)
+    per_query = 8 * (2 * k + 2)
+    if nq * per_query > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(nq, DUMP_BYTES // per_query, replace=False))
+    counts = counts[rows].astype(np.int64)
+    live = np.arange(k)[None, :] < counts[:, None]
+    values = metric.to_float(np.where(live, bits[rows].view(np.uint64), np.uint64(0))).astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("ordinals", np.where(live, ords[rows].astype(np.float64), -1.0)),
+                      ("distances", np.where(live, values, np.inf)),
+                      ("counts", counts.astype(np.float64)), ("query_rows", rows.astype(np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
 
 
 def config_dict(a, n_gpus):
@@ -394,7 +427,7 @@ def run_ours(a):
     dev_ms, wall_ms = float(t[0]), float(t[1])
     ms_per_step = dev_ms / a.steps
     value = nq * a.steps / (dev_ms / 1e3)
-    d_last = (d_ord.cpu(), d_bits.cpu())
+    d_last = (d_ord.cpu(), d_bits.cpu(), d_cnt.cpu())
 
     # ---- end-to-end leg through the host-buffer C ABI call: H2D of the rank's query slice, D2H of its ids/distances/counts ----
     for b in range(min(3, a.warmup)):
@@ -476,6 +509,16 @@ def run_ours(a):
             cpu = {"value": done_q / spent, "unit": "queries/s", "cores": cores, "kind": "port",
                    "sample": f"{done_q} queries ({done_q // nq} of the run's {nb} batches), {spent:.1f}s on {cores} threads; "
                              "restated reference, in-memory forest (storage engine excluded)"}
+
+    if a.dump_outputs:
+        outs = [t.numpy() for t in d_last]
+        if G > 1:   # every rank holds its slice of the batch; slice_bounds orders the slices by rank
+            parts = [None] * G if rank == 0 else None
+            dist.gather_object(outs, parts, dst=0)
+            if rank == 0:
+                outs = [np.concatenate([p[i] for p in parts]) for i in range(3)]
+        if rank == 0:
+            dump_outputs(a.dump_outputs, metric, *outs)
 
     per_rank = None
     if G > 1:   # per-rank phase times (ms per step): the step time is the max over ranks, these show where it goes
