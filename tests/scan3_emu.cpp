@@ -472,7 +472,7 @@ extern "C" __attribute__((visibility("default"))) int emu_project3(int blocks, i
     return (int)counter;
 }
 
-extern "C" __attribute__((visibility("default"))) void emu_scan3_layout(int nst, int dim, int qcap, uint32_t* out8) {
-    const zb::T3Layout l = zb::t3_layout(nst, (dim + 15) / 16 * 16, qcap, 1);
+extern "C" __attribute__((visibility("default"))) void emu_scan3_layout(int nst, int dim, int qcap, int kr, uint32_t* out8) {
+    const zb::T3Layout l = zb::t3_layout(nst, (dim + 15) / 16 * 16, qcap, kr);
     out8[0] = l.stage; out8[1] = l.queries; out8[2] = l.sums; out8[3] = l.lists; out8[4] = l.meta; out8[5] = l.info; out8[6] = l.bars; out8[7] = l.total;
 }

@@ -54,7 +54,7 @@ def assert_search_equal(ix, orc, queries, k, nthreads=8):
 
 
 # ------------------------------------------------------------------------------------------ arithmetic
-@pytest.mark.parametrize("dim", [4, 16, 20, 384, 768])
+@pytest.mark.parametrize("dim", [4, 16, 20, 384, 768, 1024, 4096, 8192])
 @pytest.mark.parametrize("mid,mname", METRICS)
 def test_metric_bits_exact(dim, mid, mname):
     rng = np.random.default_rng(dim + mid)
@@ -72,7 +72,7 @@ def test_metric_bits_exact(dim, mid, mname):
     assert metric_obj(mname).distance(a[7], b[7]) == int(exp[7])
 
 
-@pytest.mark.parametrize("dim", [16, 40, 384, 768])
+@pytest.mark.parametrize("dim", [16, 40, 384, 768, 1024, 4096, 8192])
 def test_point_is_above_bit_exact_including_adversarial(dim):
     rng = np.random.default_rng(dim)
     n = 4096

@@ -45,7 +45,7 @@ def assert_search_equal(ix, orc, queries, k, nthreads=8):
         assert np.all(ords[q, c:] == np.iinfo(np.uint64).max)
 
 
-@pytest.mark.parametrize("dim", [1, 3, 4, 5, 16, 20, 384, 768])
+@pytest.mark.parametrize("dim", [1, 3, 4, 5, 16, 20, 384, 768, 1024, 4096, 8192])
 def test_scalar_metric_bits_exact(dim):
     rng = np.random.default_rng(50 + dim)
     a, b = adversarial(rng, 700, dim)

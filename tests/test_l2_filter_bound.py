@@ -47,8 +47,10 @@ def check_pairs(a, b):
     return float((err[usable] / eq[usable]).max())
 
 
-@pytest.mark.parametrize("dim", [1, 7, 16, 48, 100, 384, 768, 1000])
+@pytest.mark.parametrize("dim", [1, 7, 16, 48, 100, 384, 768, 1000, 1024, 1536, 2048, 3072, 4096, 4672])
 def test_bound_on_random_and_cancelling_pairs(dim):
+    """Up to 4672 dimensions: the widest row for which the fused kernel (and with it the filter) still fits in shared memory
+    (test_scan3.py::test_tile_config_regimes)."""
     rng = np.random.default_rng(dim)
     worst = 0.0
     for scale in (1.0, 1e-3, 1e3, 1e-15, 1e15):

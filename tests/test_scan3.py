@@ -6,7 +6,8 @@ tree_result (/root/reference/src/database/index/lsh.rs:299-331) with Metric::dis
 What this covers without a GPU: the ring protocol (full / empty / tile-info / query barriers: a missing wait reads stale
 data because copies land late, an extra arrival aborts), the 16-lane fold over the half-warp and which thread ends up with
 which row, the transposition through shared memory, list insertion with ties and tombstones, partial row blocks, partial
-query tiles (QH = 1 .. 8), dim % 48 != 0 and dim % 16 != 0, and the shared per-query bound."""
+query tiles (QH = 1 .. 8), dim % 48 != 0 and dim % 16 != 0, and the shared per-query bound; the shared-memory layout and
+the tile capacity (16, 8 or 4 queries) the launch code picks as rows grow, and the kernel body run at each capacity."""
 import ctypes as C
 import os
 import subprocess
@@ -28,16 +29,47 @@ def emu(tmp_path_factory, request):
     TW = 8 (eight math warps per team, 8 rows of a block each: 640 threads; what the library launches for n' > 32)."""
     kc, epw, tw = request.param
     out = str(tmp_path_factory.mktemp("s3") / f"libscan3_emu_kc{kc}_epw{epw}_tw{tw}.so")
+    build_emu(out, kc, epw)
+    return load_emu(out, kc, epw, tw)
+
+
+def build_emu(out, kc=3, epw=0):
     subprocess.check_call(["g++", "-O1", "-std=c++20", "-ffp-contract=off", "-fno-fast-math", "-fPIC", "-shared", "-pthread",
                            f"-DT3_KC={kc}", f"-DT3_EPW={epw}", "-g", "-rdynamic", "-fvisibility=hidden", "-Wl,-Bsymbolic", "-o", out,
                            os.path.join(HERE, "scan3_emu.cpp")])
-    L = C.CDLL(out)
+
+
+def load_emu(path, kc=3, epw=0, tw=4):
+    L = C.CDLL(path)
     assert L.emu_scan3_set_team_warps(tw) == 0               # the kernel body's TW (a template parameter: both shapes are in every build)
     L.variant = (kc, epw, tw)
     L.emu_scan3.restype = C.c_int
     L.emu_scan3.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_uint64] + [C.c_void_p] * 7 + \
                            [C.c_uint32] + [C.c_void_p] * 12
+    L.emu_scan3_layout.restype = None
+    L.emu_scan3_layout.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
     return L
+
+
+# ---- shared-memory layout and the (query capacity, ring depth) the launch code picks -------------------------------------
+OPTIN_B200 = 232_448          # cudaDevAttrMaxSharedMemoryPerBlockOptin of a B200 (227 KB)
+LAYOUT_FIELDS = ("stage", "queries", "sums", "lists", "meta", "info", "bars", "total")
+
+
+def scan3_layout(emu, nst, dim, qcap, kr):
+    out = np.zeros(8, np.uint32)
+    emu.emu_scan3_layout(nst, dim, qcap, kr, out.ctypes.data)
+    return dict(zip(LAYOUT_FIELDS, (int(x) for x in out)))
+
+
+def t3_config(emu, dim, kr, optin=OPTIN_B200):
+    """zb_scan.cu t3_config over the header's t3_layout: the largest tile (16, 8, then 4 queries) that leaves at least 3 ring
+    stages for two teams + 1024 B, with the deepest ring that fits; None where the fused kernel does not fit at all."""
+    for qcap in (16, 8, 4):
+        for nst in range(8, 2, -1):
+            if 2 * scan3_layout(emu, nst, dim, qcap, kr)["total"] + 1024 <= optin:
+                return qcap, nst
+    return None
 
 
 def canonical_sq_norm(x):
@@ -202,6 +234,95 @@ def test_small_query_capacity_and_deep_ring(emu):
     entries, ent_off, v_np, _ = run_emu(emu, case, zo.COSINE, top_k=0xFFFFFFFF, tq=8, qcap=8, nst=6, blocks=1)
     for v in range(case["v_leaf"].size):
         assert np.array_equal(entries[ent_off[v]:ent_off[v + 1]], expected_visit(case, zo.COSINE, v, int(v_np[v]))), v
+
+
+def test_tile_config_regimes(emu):
+    """Which tile shape the launch code picks as rows grow, and that every shape it can pick is a sound layout: regions in
+    order without overlap, each as large as the kernel addresses it, TMA / bulk-copy destinations on 128 B, the tile info on
+    16 B, mbarriers on 8 B, and two teams + 1024 B of alignment slack within the 227 KB a block may opt into."""
+    picked = {}
+    for kr in (1, 4):
+        for dimp in range(16, 6001, 16):
+            picked[kr, dimp] = cfg = t3_config(emu, dimp, kr)
+            if cfg is None:
+                continue
+            qcap, nst = cfg
+            lay = scan3_layout(emu, nst, dimp, qcap, kr)
+            need = dict(stage=nst * 64 * emu.variant[0] * 16 * 4,
+                        queries=(qcap * dimp + 16) * 4,              # two regions of qcap / 2 queries, the second 64 B further
+                        sums=2 * qcap * 64 * 4, lists=qcap * 3 * kr * 32 * 4, meta=5 * qcap * 4,
+                        info=2 * 32, bars=(2 * 8 + 8) * 8)
+            names = LAYOUT_FIELDS[:-1]
+            assert lay["stage"] == 0
+            for a, b in zip(names, names[1:] + ("total",)):
+                assert lay[b] - lay[a] >= need[a], (kr, dimp, cfg, a, lay)
+            for f in ("stage", "queries", "sums", "total"):
+                assert lay[f] % 128 == 0, (kr, dimp, cfg, f, lay)
+            assert lay["info"] % 16 == 0 and lay["bars"] % 8 == 0, (kr, dimp, cfg, lay)
+            assert 2 * lay["total"] + 1024 <= OPTIN_B200
+    for kr in (1, 4):                                   # the ring only grows shallower inside a capacity
+        seq = [picked[kr, d] for d in range(16, 6001, 16) if picked[kr, d]]
+        assert all(a[0] > b[0] or (a[0] == b[0] and a[1] >= b[1]) for a, b in zip(seq, seq[1:])), kr
+    if emu.variant[0] != 3:
+        return                                                  # the regimes below are those of the 12 KB stage the library ships
+    cap = lambda kr, d: picked[kr, d] and picked[kr, d][0]
+    assert picked[1, 16] == (16, 8) and picked[1, 992] == (16, 3)
+    assert cap(1, 992) == 16 and cap(1, 1008) == 8              # n' <= 32: 16-query tiles up to 992 floats per row
+    assert cap(1, 2208) == 8 and cap(1, 2224) == 4
+    assert cap(1, 4672) == 4 and picked[1, 4688] is None        # beyond: quad_tile / score_pairs
+    assert cap(4, 704) == 16 and cap(4, 720) == 8               # n' <= 128
+    assert cap(4, 1920) == 8 and cap(4, 1936) == 4
+    assert cap(4, 4384) == 4 and picked[4, 4400] is None
+    for dim, qcap, nst1, nst4 in SMALL_TILES:
+        assert picked[1, dim] == (qcap, nst1) and picked[4, dim] == (qcap, nst4)
+
+
+# (dim, qcap, ring depth for n' <= 32, ring depth for n' <= 128): what the launch code picks at these row lengths
+SMALL_TILES = [(1040, 8, 6, 5), (2240, 4, 6, 5)]
+
+
+def check_small_tiles(emu, dim, qcap, nst, kr):
+    """The kernel body at a tile capacity below 16 with the ring depth picked for that row length: tiles of every size 1 .. qcap
+    (one leaf per size, one with two full tiles and a single query), tombstones, exact duplicate rows, a query equal to a
+    stored row, partial row blocks; every visit's list exact for the three exact metrics and (n' <= 32) for L2 / L2 squared
+    through the dot-product filter and its second pass; then n' = top_k everywhere, so the shared per-query bound is
+    published and read, and the per-query answer must not change."""
+    rng = np.random.default_rng(dim + 10 * qcap + kr)
+    visits = list(range(1, qcap + 1)) + [2 * qcap + 1]
+    leaf_lens = [1, 63, 64, 65, 130, 17, 70, 128, 129][:len(visits) - 1] + [150]
+    np_max = 32 if kr == 1 else 128
+    case = build_case(rng, dim, leaf_lens, 2 * qcap + 3, visits, np_max=np_max, tomb_frac=0.15)
+    if kr != 1:
+        case["v_np"][:4] = [128, 127, 100, 33]
+    lo = int(case["leaf_off"][-2])                              # last leaf: a group of near copies of one row (the filter's cancellation)
+    for i in range(1, 25):
+        case["rows"][lo + i] = case["rows"][lo]
+        case["rows"][lo + i, i] = np.nextafter(case["rows"][lo, i], F32(np.inf) if i % 2 else F32(-np.inf), dtype=F32)
+    case["queries"][1] = case["rows"][lo]
+    for metric in (zo.COSINE, zo.L2SQ, zo.L2):
+        entries, ent_off, v_np, _ = run_emu(emu, case, metric, top_k=0xFFFFFFFF, tq=qcap, qcap=qcap, nst=nst, kr=kr)
+        check_every_visit(case, metric, entries, ent_off, v_np)
+    if kr == 1:                                                 # the filter takes n' <= 16
+        fcase = dict(case, v_np=np.minimum(case["v_np"], 16))
+        entries, ent_off, v_np, _ = run_emu(emu, fcase, zo.L2SQ, top_k=0xFFFFFFFF, tq=qcap, qcap=qcap, nst=nst, l2_filter=True)
+        check_every_visit(fcase, zo.L2SQ, entries, ent_off, v_np)
+    k = 10 if kr == 1 else 100
+    for filt in ((False, True) if kr == 1 else (False,)):
+        entries, ent_off, _, gthr = run_emu(emu, case, zo.L2, top_k=k, tq=qcap, qcap=qcap, nst=nst, kr=kr, same_np=k, blocks=2,
+                                            l2_filter=filt)
+        assert (gthr != SENT).any()
+        for q in range(case["queries"].shape[0]):
+            got, exp = [], []
+            for v in np.nonzero(case["v_q"] == q)[0]:
+                got += [tuple(x) for x in entries[ent_off[v]:ent_off[v + 1]] if x[1] != SENT]
+                exp += [tuple(x) for x in expected_visit(case, zo.L2, v, k)]
+            assert sorted(set(got))[:k] == sorted(set(exp))[:k], (filt, q)
+
+
+@pytest.mark.parametrize("kr", [1, 4])
+@pytest.mark.parametrize("dim,qcap,nst1,nst4", SMALL_TILES, ids=[f"{d}d-{q}q" for d, q, _, _ in SMALL_TILES])
+def test_small_tile_capacities(emu, dim, qcap, nst1, nst4, kr):
+    check_small_tiles(emu, dim, qcap, nst1 if kr == 1 else nst4, kr)
 
 
 @pytest.mark.parametrize("dim,H,n,tq", [(48, 16, 200, 16), (100, 37, 333, 16), (64, 5, 70, 16), (200, 24, 150, 8)])

@@ -1427,6 +1427,8 @@ void seq_tile_scan(ScanWorkspace& ws, const ForestView& f, u32 metric, int power
     tp.stats = reinterpret_cast<u64*>(ws.counters.p + 4);
     tp.power = power;
     tp.pf_lines = prefetch_lines < 0 ? 0 : (prefetch_lines > 64 ? 64 : prefetch_lines);
+    // the opt-in is set whatever the size: the kernel's static shared memory counts against the 48 KB default too, so rows of
+    // 1536 floats (exactly 48 KB of queries) failed to launch without it
     const size_t smem = (size_t)SQ_TQ * f.dimp * 4;
     const int grid = sms * SQ_CTAS_PER_SM;
     if (!ws.ev0) {
@@ -1436,8 +1438,7 @@ void seq_tile_scan(ScanWorkspace& ws, const ForestView& f, u32 metric, int power
     ZB_CUDA(cudaEventRecord(ws.ev0, s));
 #define ZB_SQ_CALL(C)                                                                                                        \
     do {                                                                                                                     \
-        if (smem > 48 * 1024)                                                                                                \
-            ZB_CUDA(cudaFuncSetAttribute(seq_tile_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));        \
+        ZB_CUDA(cudaFuncSetAttribute(seq_tile_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
         seq_tile_kernel<C><<<grid, SQ_THREADS, smem, s>>>(f, tp);                                                            \
     } while (0)
     switch (metric) {
@@ -1527,7 +1528,7 @@ void quad_tile_scan(ScanWorkspace& ws, const ForestView& f, u32 metric, const fl
     tp.pair_key = pair_key;
     tp.queries = d_q;
     tp.stats = reinterpret_cast<u64*>(ws.counters.p + 4);
-    const size_t smem = (size_t)8 * f.dimp * 4;
+    const size_t smem = (size_t)8 * f.dimp * 4;   // opt-in set whatever the size, as for seq_tile_kernel (static shared memory)
     const int grid = sms * 2;
     if (!ws.ev0) {
         ZB_CUDA(cudaEventCreate(&ws.ev0));
@@ -1536,8 +1537,7 @@ void quad_tile_scan(ScanWorkspace& ws, const ForestView& f, u32 metric, const fl
     ZB_CUDA(cudaEventRecord(ws.ev0, s));
 #define ZB_QT_CALL(M)                                                                                                    \
     do {                                                                                                                 \
-        if (smem > 48 * 1024)                                                                                            \
-            ZB_CUDA(cudaFuncSetAttribute(quad_tile_kernel<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
+        ZB_CUDA(cudaFuncSetAttribute(quad_tile_kernel<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));       \
         quad_tile_kernel<M><<<grid, QT_THREADS, smem, s>>>(f, tp);                                                       \
     } while (0)
     if (metric == 0) ZB_QT_CALL(0);
