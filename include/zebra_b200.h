@@ -165,6 +165,23 @@ int zb_index_search_slice_device(zb_index* index, uint64_t nq_total, const float
  * call whose pointer was not announced uploads its queries itself, and results never depend on it. */
 int zb_index_search_prefetch(zb_index* index, uint64_t n, const float* queries);
 
+/* Exact (brute-force) search: for each query the top_k smallest (DistanceUnit bits, ordinal) pairs over EVERY live (not
+ * removed) row of the index, in the order LSHIndex::search sorts its candidates (lsh.rs:557-564), literal cosine of quirk
+ * Q4 included -- the ground truth the LSH search's recall is measured against.  Output layout, 0xFF tail fill, out_counts
+ * and the NULL-able outputs are those of zb_index_search_batch / zb_index_search_batch_device; top_k = 0 gives counts 0.
+ * Distances are bit-identical to Metric::distance of the pair, so a row both searches return carries the same bits.  The
+ * forest is not used: the scan reads the stored rows, ordinals and tombstones; an index without live rows gives counts 0.
+ * Served for metrics 0..2 with 1 <= top_k <= 128 and rows of at most 4672 padded dimensions (top_k <= 32) or 4384
+ * (top_k 33..128), the shapes of the fused leaf-tile kernel (227 KB of shared memory per block); anything else -- a scalar
+ * metric, top_k > 128, a longer row -- returns ZB_ERR_INVALID.  Queries are processed in chunks whose workspace (visit
+ * arrays, lists, the dot-product filter's candidates, a sharded call's gathered lists) stays within 256 MiB (knob
+ * "exact_budget_mb"), whatever nq is.  It leaves zb_stats alone: zb_index_stats still describes the last LSH batch.
+ * Sharded index: collective; every rank passes the same nq queries and receives the full results. */
+int zb_index_search_exact(zb_index* index, uint64_t nq, const float* queries, uint64_t top_k, uint8_t* out_ids16,
+                          uint64_t* out_ordinals, uint64_t* out_dist_bits, uint32_t* out_counts);
+int zb_index_search_exact_device(zb_index* index, uint64_t nq, const float* d_queries, uint64_t top_k,
+                                 uint64_t* d_out_ordinals, uint64_t* d_out_dist_bits, uint32_t* d_out_counts);
+
 /* Bucket keys: the root-to-leaf sign path of Hyperplane::point_is_above decisions (lsh.rs:39-43 along
  * :350-366), MSB = root, 1 = above/right, for every (row, tree): out_keys/out_depths/out_leaves are
  * [n][num_trees] (a path longer than 64 keeps its last 64 bits; out_leaves is the leaf number of
@@ -273,7 +290,8 @@ int zb_index_stream(zb_index* index, void** out_stream);
  * "select_variant", "bm_stage_mb", "single_exchange", "p2p_queries",
  * "l2_filter" (L2 / L2 squared with top_k <= 16 scored through the dot product + exact second pass: 0 off, 1 adaptive = default,
  *              2 always), "long_list_warps" (math warps per team of the fused scan for top_k > 32: 8 = default, 4),
- * "plan_tail" (count-cascade walkers re-walked by the latency-optimised tail kernel: 1 = default, 0)}. */
+ * "plan_tail" (count-cascade walkers re-walked by the latency-optimised tail kernel: 1 = default, 0),
+ * "exact_budget_mb" (workspace of one query chunk of zb_index_search_exact*, MiB: 256 = default)}. */
 int zb_index_set_param(zb_index* index, const char* key, int64_t value);
 
 /* Sharding over the GPUs of one box: one process per GPU, each with its own index

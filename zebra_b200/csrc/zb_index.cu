@@ -188,9 +188,17 @@ struct zb_index {
     ScanWorkspace scan_ws;
     ScanWorkspace pj_ws;  // flat-table projection (project3)
     ScanWorkspace qt_ws;  // keys-only tile scan of the visits the fused kernel leaves (cosine / L2, n' > 32)
+    // exact search (zb_index_search_exact*): its own scan workspace; per-slot side arrays of the raw store, valid while
+    // ex_gen == store_gen (every path that appends or replaces rows bumps store_gen); local / gathered lists of a sharded call
+    ScanWorkspace ex_ws;
+    u64 store_gen = 0, ex_gen = ~0ull;
+    DBuf<u32> ex_iota, ex_counts;
+    DBuf<double> ex_rinv;
+    DBuf<float> ex_n2;
+    DBuf<u64> ex_loc, ex_gath, ex_nmax;
 
     // ---- knobs / stats ----
-    int64_t p_tile_min_rows = 64, p_tile_queries = 0, p_use_tile_scan = 1, p_hash_variant = 0, p_classify_variant = 0, p_seq_tile = 1, p_seq_prefetch = 0, p_flat_project = 1, p_quad_tile = 1, p_select_variant = 1, p_scan_gen = 3, p_bm_stage_mb = 2048, p_single_exchange = 1, p_p2p_queries = 1, p_l2_filter = 1, p_plan_tail = 1;
+    int64_t p_tile_min_rows = 64, p_tile_queries = 0, p_use_tile_scan = 1, p_hash_variant = 0, p_classify_variant = 0, p_seq_tile = 1, p_seq_prefetch = 0, p_flat_project = 1, p_quad_tile = 1, p_select_variant = 1, p_scan_gen = 3, p_bm_stage_mb = 2048, p_single_exchange = 1, p_p2p_queries = 1, p_l2_filter = 1, p_plan_tail = 1, p_exact_budget_mb = 256;
     zb_stats st{};
 
     ForestView view() const {
@@ -309,7 +317,8 @@ struct zb_index {
         ord.ensure(ncap, n_slots, stream, true);
         row_norm.ensure(ncap, n_slots, stream, true);
         size_t old_words = tomb.cap;
-        tomb.ensure(ncap / 32 + 1, (n_slots + 31) / 32, stream, true);
+        // + 3: the fused scan's exact mode reads three words from the first word of every 64-row block
+        tomb.ensure(ncap / 32 + 3, (n_slots + 31) / 32, stream, true);
         (void)old_words;
         // slot_leaf is [T][stride]: re-stride
         DBuf<u32> nsl;
@@ -345,6 +354,22 @@ struct zb_index {
         h_tomb.resize(h_tomb.size() + n_local, 0);
         n_slots += n_local;
         n_live += n_local;
+        ++store_gen;
+    }
+    // exact search: identity member list, and per slot 1/sqrt(|row|^2) (cosine) or canonical |row|^2 (L2, L2 squared)
+    void ensure_exact_side() {
+        if (ex_gen == store_gen) return;
+        const u64 n = n_slots ? n_slots : 1;
+        ex_iota.ensure(n);
+        launch_iota_u32(ex_iota.p, n_slots, 0u, stream);
+        if (opt.metric == ZB_METRIC_COSINE) {
+            ex_rinv.ensure(n);
+            launch_rinv(rows.p, n_slots, dimp, ex_rinv.p, stream);
+        } else {
+            ex_n2.ensure(n);
+            launch_n2(rows.p, n_slots, dimp, ex_n2.p, stream);
+        }
+        ex_gen = store_gen;
     }
 
     // ---------------------------------------------------------------- forest upload helpers
@@ -1300,6 +1325,66 @@ static void search_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64
     ix->st.last_total_launches += scan_launches + 5 + (sharded ? 1 : 0) + ((ix->scan_ws.seq_launched || ix->qt_ws.seq_launched) ? 6 : 0);
 }
 
+// Exact search (zb_index_search_exact*): the top_k smallest (bits, ordinal) over every live row of the raw store.  Each rank
+// scans the rows it owns; a sharded call allgathers the ranks' per-query lists and merges them (the same exchange as the
+// unsliced search).  Queries go in chunks that keep the workspace within the exact_budget_mb knob; the plan comes from the
+// largest row count of all ranks, so every rank runs the same sequence of collectives.
+static void exact_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64* d_out_ord, u64* d_out_bits, u32* d_out_counts) {
+    cudaStream_t s = ix->stream;
+    if (!nq) return;
+    if (!top_k) {
+        ZB_CUDA(cudaMemsetAsync(d_out_counts, 0, nq * 4, s));
+        return;
+    }
+    const u32 G = ix->G;
+    const bool sharded = G > 1;
+    u64 n_max = ix->n_slots;
+    if (sharded) {
+        ix->ex_nmax.ensure(1);
+        ZB_CUDA(cudaMemcpyAsync(ix->ex_nmax.p, &n_max, 8, cudaMemcpyHostToDevice, s));
+        ix->nccl.allreduce(ix->ex_nmax.p, 1, Nccl::U64, Nccl::MAX, s);
+        ZB_CUDA(cudaMemcpyAsync(&n_max, ix->ex_nmax.p, 8, cudaMemcpyDeviceToHost, s));
+        ix->sync();
+    }
+    const u32 metric = ix->opt.metric;
+    // L2 / L2 squared with short lists go through the dot-product filter, as in the LSH search (DESIGN 3.8: measured on config 2)
+    const bool filt = (metric == ZB_METRIC_L2SQ || metric == ZB_METRIC_L2) && top_k <= ZB_L2_FILTER_MAX_K && ix->dimp >= 128;
+    ix->ensure_exact_side();
+    // per query: q_rinv / q_n2 / shared bound, and (sharded) its local lists plus the G gathered ones
+    const u64 per_query = 24 + (sharded ? 16 * top_k * (G + 1) + 4 : 0);
+    const ExactPlan p = exact_plan(n_max, nq, ix->dimp, (u32)top_k, filt, per_query, (u64)ix->p_exact_budget_mb << 20);
+    ForestView store = ix->view();
+    store.members = ix->ex_iota.p;
+    BucketMajor bm;
+    bm.rows = ix->rows.p;
+    bm.tomb = ix->tomb.p;
+    bm.rinv = metric == ZB_METRIC_COSINE ? ix->ex_rinv.p : nullptr;
+    bm.n2 = filt ? ix->ex_n2.p : nullptr;
+    alignas(64) unsigned char tmap[128];
+    if (ix->n_slots) make_row_tile_map(tmap, ix->rows.p, ix->n_slots, ix->dimp, 64, tile_scan_box_floats(3));
+    bm.tmap3 = tmap;
+    bm.positions = ix->n_slots;
+    for (u64 c0 = 0; c0 < nq; c0 += p.chunk) {
+        const u64 c = std::min<u64>(p.chunk, nq - c0);
+        const float* q = d_q + c0 * (u64)ix->dimp;
+        if (!sharded) {
+            exact_scan3(ix->ex_ws, store, bm, ix->n_slots, metric, q, (u32)c, p.range_rows, (u32)top_k, filt, d_out_ord + c0 * top_k,
+                        d_out_bits + c0 * top_k, d_out_counts + c0, s);
+            continue;
+        }
+        const u64 nsk = c * top_k;   // [ord nsk | bits nsk] per rank, the layout merge_gathered reads
+        ix->ex_loc.ensure(2 * p.chunk * top_k);
+        ix->ex_gath.ensure(2 * p.chunk * top_k * G);
+        ix->ex_counts.ensure(p.chunk);
+        exact_scan3(ix->ex_ws, store, bm, ix->n_slots, metric, q, (u32)c, p.range_rows, (u32)top_k, filt, ix->ex_loc.p,
+                    ix->ex_loc.p + nsk, ix->ex_counts.p, s);
+        ix->nccl.allgather(ix->ex_loc.p, ix->ex_gath.p, 2 * nsk * 8, s);
+        launch_merge_gathered((u32)c, (u32)c, (u32)top_k, G, ix->ex_gath.p, d_out_ord + c0 * top_k, d_out_bits + c0 * top_k,
+                              d_out_counts + c0, s);
+    }
+    ix->sync();
+}
+
 static const float* stage_queries_device(zb_index* ix, const float* d_q, u64 nq) {
     if (ix->dim == ix->dimp && ((uintptr_t)d_q & 15) == 0) return d_q;
     ix->q_stage.ensure(nq * (u64)ix->dimp);
@@ -1730,7 +1815,7 @@ int zb_index_no_trees(zb_index* ix, int* out) {
 // Batches beyond 131072 queries are cut into chunks (walker count < 2^31, bounded workspaces).  sliced: see search_device;
 // the chunks of a sliced call are chunks of the whole batch, so every rank sees the same sequence of collectives.
 static void search_entry_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64* d_out_ord, u64* d_out_bits,
-                                u32* d_out_counts, bool sliced) {
+                                u32* d_out_counts, bool sliced, bool exact = false) {
     ix->use_device();
     const u64 G = ix->G;
     sliced = sliced && G > 1;
@@ -1744,7 +1829,8 @@ static void search_entry_device(zb_index* ix, u64 nq, const float* d_q, u64 top_
             mine = std::min<u64>(nqp, c - lo);
         }
         const float* q = stage_queries_device(ix, d_q + in_off * (u64)ix->dim, mine);
-        search_device(ix, c, q, top_k, d_out_ord + in_off * top_k, d_out_bits + in_off * top_k, d_out_counts + in_off, sliced);
+        if (exact) exact_device(ix, c, q, top_k, d_out_ord + in_off * top_k, d_out_bits + in_off * top_k, d_out_counts + in_off);
+        else search_device(ix, c, q, top_k, d_out_ord + in_off * top_k, d_out_bits + in_off * top_k, d_out_counts + in_off, sliced);
         in_off += mine;
     }
     ix->sync();
@@ -1771,7 +1857,7 @@ int zb_index_search_slice_device(zb_index* ix, uint64_t nq_total, const float* d
 
 // Host buffers in, host buffers out.  sliced: `queries` and the outputs hold this rank's slices only.
 static void search_entry_host(zb_index* ix, u64 nq, const float* queries, u64 top_k, uint8_t* out_ids16, u64* out_ordinals,
-                              u64* out_bits, u32* out_counts, bool sliced) {
+                              u64* out_bits, u32* out_counts, bool sliced, bool exact = false) {
     ix->use_device();
     cudaStream_t s = ix->stream;
     const u64 G = ix->G;
@@ -1787,7 +1873,7 @@ static void search_entry_host(zb_index* ix, u64 nq, const float* queries, u64 to
             mine = std::min<u64>(nqp, c - lo);
         }
         bool staged = false;
-        if (c0 == 0 && mine) {  // announced by zb_index_search_prefetch: the rows are (being) copied on the copy stream
+        if (c0 == 0 && mine && !exact) {  // announced by zb_index_search_prefetch: the rows are (being) copied on the copy stream
             for (auto& p : ix->pf)
                 if (p.host == queries && p.rows >= mine && nq <= chunk) {
                     ZB_CUDA(cudaStreamWaitEvent(s, p.done, 0));
@@ -1811,7 +1897,8 @@ static void search_entry_host(zb_index* ix, u64 nq, const float* queries, u64 to
         ix->o_ord.ensure(mine * top_k + 1);
         ix->o_bits.ensure(mine * top_k + 1);
         ix->o_counts2.ensure(mine + 1);
-        search_device(ix, c, ix->q_stage.p, top_k, ix->o_ord.p, ix->o_bits.p, ix->o_counts2.p, sliced);
+        if (exact) exact_device(ix, c, ix->q_stage.p, top_k, ix->o_ord.p, ix->o_bits.p, ix->o_counts2.p);
+        else search_device(ix, c, ix->q_stage.p, top_k, ix->o_ord.p, ix->o_bits.p, ix->o_counts2.p, sliced);
         if (!out_ordinals && out_ids16) ord_tmp.resize(mine * top_k);
         u64* ords = out_ordinals ? out_ordinals + in_off * top_k : ord_tmp.data();
         if (top_k && mine) {
@@ -1838,6 +1925,34 @@ int zb_index_search_batch(zb_index* ix, uint64_t nq, const float* queries, uint6
     ZB_REQUIRE(top_k <= ZB_MAX_TOPK, ZB_ERR_INVALID, "top_k %llu exceeds %d", (unsigned long long)top_k, ZB_MAX_TOPK);
     std::lock_guard<std::mutex> lk(ix->mu);
     search_entry_host(ix, nq, queries, top_k, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, false);
+    ZB_API_END
+}
+static void exact_check(zb_index* ix, u64 top_k) {
+    ZB_REQUIRE(ix->opt.metric <= ZB_METRIC_L2, ZB_ERR_INVALID, "exact search serves cosine, L2 squared and L2, not metric %u",
+               ix->opt.metric);
+    ZB_REQUIRE(top_k <= ZB_EXACT_MAX_K, ZB_ERR_INVALID, "exact search: top_k %llu exceeds %d", (unsigned long long)top_k,
+               ZB_EXACT_MAX_K);
+    ix->use_device();
+    ZB_REQUIRE(tile_scan3_supported(ix->dimp, top_k ? (u32)top_k : 1u), ZB_ERR_INVALID,
+               "exact search: %d dimensions exceed the fused scan's limit for top_k %llu", ix->dim, (unsigned long long)top_k);
+    if (ix->G > 1) ZB_REQUIRE(ix->comm_ready, ZB_ERR_STATE, "sharded index used before zb_index_comm_init");
+}
+int zb_index_search_exact(zb_index* ix, uint64_t nq, const float* queries, uint64_t top_k, uint8_t* out_ids16,
+                          uint64_t* out_ordinals, uint64_t* out_bits, uint32_t* out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && (queries || !nq) && ((out_bits && out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
+    std::lock_guard<std::mutex> lk(ix->mu);
+    exact_check(ix, top_k);
+    search_entry_host(ix, nq, queries, top_k, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, false, true);
+    ZB_API_END
+}
+int zb_index_search_exact_device(zb_index* ix, uint64_t nq, const float* d_q, uint64_t top_k, uint64_t* d_out_ord,
+                                 uint64_t* d_out_bits, uint32_t* d_out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && (d_q || !nq) && ((d_out_ord && d_out_bits && d_out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
+    std::lock_guard<std::mutex> lk(ix->mu);
+    exact_check(ix, top_k);
+    search_entry_device(ix, nq, d_q, top_k, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, false, true);
     ZB_API_END
 }
 int zb_index_search_prefetch(zb_index* ix, uint64_t n, const float* queries) {
@@ -2030,6 +2145,7 @@ static void clear_locked(zb_index* ix) {
     ix->sync();
     ix->clear_forest();
     ix->n_slots = ix->n_live = ix->total_rows = 0;
+    ++ix->store_gen;
     ix->h_ord.clear();
     ix->h_tomb.clear();
     ix->flat_bits = 0;
@@ -2319,6 +2435,10 @@ int zb_index_set_param(zb_index* ix, const char* key, int64_t value) {
     else if (k == "flat_project") ix->p_flat_project = value;  // flat tables: 1 = dense projection + ballot packing (default), 0 = the generic tree walk
     else if (k == "l2_filter") { ix->p_l2_filter = value; ix->filter_backoff = 0; }  // L2 / L2 squared through the dot-product filter + exact second pass: 0 off, 1 adaptive (default), 2 always
     else if (k == "long_list_warps") { ZB_REQUIRE(value == 4 || value == 8, ZB_ERR_INVALID, "long_list_warps is 4 or 8"); ix->scan_ws.long_list_warps = (int)value; }  // fused scan with n' > 32: math warps per team
+    else if (k == "exact_budget_mb") {  // exact search: workspace of one query chunk, MiB (default 256)
+        ZB_REQUIRE(value >= 1 && value <= (1 << 20), ZB_ERR_INVALID, "exact_budget_mb out of range");
+        ix->p_exact_budget_mb = value;
+    }
     else if (k == "plan_tail") ix->p_plan_tail = value;  // plan walk: 1 = cascade walkers go to the latency-optimised tail kernel (default), 0 = one kernel
     else if (k == "p2p_queries") ix->p_p2p_queries = value;  // sliced search: 1 = query slices pushed into the peers' buffers over NVLink (CUDA IPC; default), 0 = NCCL
     else if (k == "single_exchange") ix->p_single_exchange = value;  // sliced search: 1 = query slices ride in the visit-record allgather (default), 0 = their own allgather first

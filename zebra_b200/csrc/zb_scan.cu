@@ -982,6 +982,9 @@ bool tile_scan3_supported(int dimp, u32 top_k) {
     int nst, qcap;
     return top_k >= 1 && top_k <= T3_KL * T3_KR_MAX && t3_config(dimp, t3_kr(top_k), &nst, &qcap);
 }
+static void t3_launch(ScanWorkspace& ws, const ForestView& f, const BucketMajor& bm, u32 metric, const float* d_q, const double* d_q_rinv,
+                      u32 nq, u32 nv, const u32* v_leaf, const u32* v_np, const u32* v_q, const u32* v_ent_off, Entry* entries, u32 top_k,
+                      int kr, int nst, int qcap, int sms, const u32* ntiles, const u32* nvisits, cudaStream_t s);
 
 void tile_scan3(ScanWorkspace& ws, const ForestView& f, const BucketMajor& bm, u32 metric, const float* d_q, const double* d_q_rinv,
                 u32 nq, u32 nv, const u32* v_leaf, const u32* v_np, const u32* v_q, const u32* v_ent_off, u64* v_pair_len,
@@ -997,7 +1000,6 @@ void tile_scan3(ScanWorkspace& ws, const ForestView& f, const BucketMajor& bm, u
     int dev = 0, sms = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const size_t smem = t3_smem_bytes(nst, f.dimp, qcap, kr);
 
     ws.leaf_count.ensure(nleaves + 1);
     ws.leaf_start.ensure(nleaves + 1);
@@ -1047,6 +1049,16 @@ void tile_scan3(ScanWorkspace& ws, const ForestView& f, const BucketMajor& bm, u
                                                                   ws.tile_leaf.p, ws.tile_first.p, ws.tile_cnt.p, f.leaf_len,
                                                                   (u64)f.dimp * 4ull, reinterpret_cast<u64*>(ws.counters.p + 4) + 3);
     }
+    t3_launch(ws, f, bm, metric, d_q, d_q_rinv, nq, nv, v_leaf, v_np, v_q, v_ent_off, entries, top_k, kr, nst, qcap, sms,
+              ws.tile_start.p + nleaves, ws.leaf_start.p + nleaves, s);
+}
+
+// The fused kernel (and the filter's second pass) over the tiles in ws.tile_leaf / tile_first / tile_cnt (*ntiles of them) and
+// the visits in ws.order (*nvisits of them), both device scalars.
+static void t3_launch(ScanWorkspace& ws, const ForestView& f, const BucketMajor& bm, u32 metric, const float* d_q, const double* d_q_rinv,
+                      u32 nq, u32 nv, const u32* v_leaf, const u32* v_np, const u32* v_q, const u32* v_ent_off, Entry* entries, u32 top_k,
+                      int kr, int nst, int qcap, int sms, const u32* ntiles, const u32* nvisits, cudaStream_t s) {
+    const size_t smem = t3_smem_bytes(nst, f.dimp, qcap, kr);
     // L2 / L2 squared with short lists: score through the dot product (half the FP32 work), exact second pass below
     const bool filt = ws.l2_filter && (metric == 1 || metric == 2) && kr == 1 && top_k <= ZB_L2_FILTER_MAX_K && bm.n2 && bm.leaf_n2max;
     ws.filtered = filt;
@@ -1068,7 +1080,7 @@ void tile_scan3(ScanWorkspace& ws, const ForestView& f, const BucketMajor& bm, u
     tp.tile_leaf = ws.tile_leaf.p;
     tp.tile_first = ws.tile_first.p;
     tp.tile_count = ws.tile_cnt.p;
-    tp.ntiles = ws.tile_start.p + nleaves;
+    tp.ntiles = ntiles;
     ws.ntiles_ptr = tp.ntiles;
     tp.tile_counter = ws.counters.p;
     tp.order = ws.order.p;
@@ -1122,7 +1134,7 @@ void tile_scan3(ScanWorkspace& ws, const ForestView& f, const BucketMajor& bm, u
         rp.bm_tomb = bm.tomb;
         rp.queries = d_q;
         rp.order = ws.order.p;
-        rp.nvisits = ws.leaf_start.p + nleaves;   // the exclusive scan's total: visits the fused kernel took
+        rp.nvisits = nvisits;
         rp.v_leaf = v_leaf;
         rp.v_np = v_np;
         rp.v_q = v_q;
@@ -1224,6 +1236,143 @@ void project3(ScanWorkspace& ws, const float* d_rows, u64 n, const float* d_coef
     ZB_CUDA(cudaFuncSetAttribute(project3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     project3_kernel<<<sms, T3Shape<4>::THREADS, smem, s>>>(tmap, f, tp);
     ZB_CUDA(cudaGetLastError());
+}
+
+// ---- exact mode: every (row range, query) pair of a plain store is a visit with n' = top_k ----
+// Visit v = q * nranges + r (query-major: query q's visits are woff[q] .. woff[q + 1], its entries v * top_k ..); tile t = range
+// t / ntq, query tile t % ntq, the queries of a range spread evenly over its ntq tiles (order is range-major).
+__global__ void ex_visits_kernel(u32 nranges, u32 nq, u32 ntq, u32 range_rows, u64 n, u32 top_k, long long* __restrict__ leaf_off,
+                                 u32* __restrict__ leaf_len, u32* __restrict__ v_leaf, u32* __restrict__ v_np, u32* __restrict__ v_q,
+                                 u32* __restrict__ order, u32* __restrict__ ent_off, u32* __restrict__ woff, u32* __restrict__ tile_leaf,
+                                 u32* __restrict__ tile_first, u32* __restrict__ tile_count, u32* __restrict__ counters) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    const u64 nv = (u64)nranges * nq, nt = (u64)nranges * ntq;
+    if (i == 0) {
+        counters[2] = (u32)nt;   // tiles
+        counters[3] = (u32)nv;   // visits (the filter's second pass)
+    }
+    if (i < nranges) {
+        leaf_off[i] = (long long)i * range_rows;
+        const u64 left = n - i * range_rows;
+        leaf_len[i] = left < range_rows ? (u32)left : range_rows;
+    }
+    if (i < nv) {
+        const u32 q = (u32)(i / nranges), r = (u32)(i - (u64)q * nranges);
+        v_leaf[i] = r;
+        v_np[i] = top_k;
+        v_q[i] = q;
+        order[(u64)r * nq + q] = (u32)i;
+    }
+    if (i <= nv) ent_off[i] = (u32)(i * top_k);
+    if (i <= nq) woff[i] = (u32)(i * nranges);
+    if (i < nt) {
+        const u32 r = (u32)(i / ntq), j = (u32)(i - (u64)r * ntq);
+        const u32 per = nq / ntq, extra = nq - per * ntq;
+        tile_leaf[i] = r;
+        tile_first[i] = r * nq + j * per + (j < extra ? j : extra);
+        tile_count[i] = per + (j < extra ? 1u : 0u);
+    }
+}
+
+static u64 ex_visit_bytes(u32 top_k, bool l2_filter) {
+    // v_leaf, v_np, v_q, ent_off, order + a tile's three words + the list; the filter's 32 candidates, cutoff and flag
+    return 5 * 4 + 3 * 4 + (u64)top_k * sizeof(Entry) + (l2_filter ? (u64)T3_KL * 8 + 4 + 1 : 0);
+}
+
+ExactPlan exact_plan(u64 n, u64 nq, int dimp, u32 top_k, bool l2_filter, u64 per_query_bytes, u64 budget_bytes) {
+    ExactPlan p;
+    int nst = 0, qcap = 0;
+    ZB_REQUIRE(t3_config(dimp, t3_kr(top_k), &nst, &qcap), ZB_ERR_INVALID, "exact search: rows of %d floats do not fit the tile kernel", dimp);
+    int dev = 0, sms = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const u64 vb = ex_visit_bytes(top_k, l2_filter);
+    n = n ? n : 1;
+    auto nranges = [&](u64 rr) { return (n + rr - 1) / rr; };
+    auto chunk = [&](u64 rr) { return std::max<u64>(1, budget_bytes / (nranges(rr) * vb + per_query_bytes + 16)); };
+    // longest ranges that still give every team several tiles (like project3); long ranges keep the visit count small
+    u64 rr = 4096;
+    while (rr > 64 && nranges(rr) * ((std::min(nq, chunk(rr)) + qcap - 1) / qcap) < (u64)sms * T3_TEAMS * 8) rr >>= 1;
+    // one query's visits must fit the budget
+    while (nranges(rr) * vb + per_query_bytes > budget_bytes && rr < (1ull << 24)) rr <<= 1;
+    p.range_rows = (u32)rr;
+    p.chunk = std::min<u64>(chunk(rr), nq ? nq : 1);
+    ZB_REQUIRE(nranges(rr) * p.chunk < (1ull << 31) && nranges(rr) * p.chunk * top_k < (1ull << 32), ZB_ERR_INVALID,
+               "exact search: too many visits in one chunk");
+    return p;
+}
+
+__global__ void ex_empty_kernel(u32 nq, u32 top_k, u64* __restrict__ out_ord, u64* __restrict__ out_bits, u32* __restrict__ out_counts) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < (u64)nq * top_k) out_ord[i] = out_bits[i] = ZB_SENTINEL;
+    if (i < nq) out_counts[i] = 0;
+}
+
+void exact_scan3(ScanWorkspace& ws, const ForestView& store, const BucketMajor& bm, u64 n, u32 metric, const float* d_q, u32 nq,
+                 u32 range_rows, u32 top_k, bool l2_filter, u64* out_ord, u64* out_bits, u32* out_counts, cudaStream_t s) {
+    ws.launched = false;
+    ws.filtered = false;
+    if (!nq || !top_k) return;
+    if (!n) {
+        const u64 tot = std::max<u64>((u64)nq * top_k, nq);
+        ex_empty_kernel<<<(u32)((tot + 255) / 256), 256, 0, s>>>(nq, top_k, out_ord, out_bits, out_counts);
+        ZB_CUDA(cudaGetLastError());
+        return;
+    }
+    int nst = 0, qcap = 0;
+    const int kr = t3_kr(top_k);
+    ZB_REQUIRE(metric <= 2 && top_k <= T3_KL * T3_KR_MAX && t3_config(store.dimp, kr, &nst, &qcap), ZB_ERR_INVALID,
+               "exact search: no fused-kernel configuration for metric %u, top_k %u, %d floats", metric, top_k, store.dimp);
+    ZB_REQUIRE(n < (1ull << 31) && range_rows % T3_RB == 0, ZB_ERR_INVALID, "exact search: %llu rows in ranges of %u",
+               (unsigned long long)n, range_rows);
+    int dev = 0, sms = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const u32 nranges = (u32)((n + range_rows - 1) / range_rows);
+    const u32 ntq = (nq + (u32)qcap - 1) / (u32)qcap;
+    const u64 nv = (u64)nranges * nq, nt = (u64)nranges * ntq;
+    ZB_REQUIRE(nv < (1ull << 31) && nv * top_k < (1ull << 32), ZB_ERR_INVALID, "exact search: too many visits in one call");
+    ws.pj_off.ensure(nranges);
+    ws.leaf_count.ensure(nranges);   // leaf_len of the ranges
+    ws.ex_leaf.ensure(nv);
+    ws.ex_np.ensure(nv);
+    ws.ex_q.ensure(nv);
+    ws.order.ensure(nv);
+    ws.ex_ent_off.ensure(nv + 1);
+    ws.ex_woff.ensure((u64)nq + 1);
+    ws.tile_leaf.ensure(nt);
+    ws.tile_first.ensure(nt);
+    ws.tile_cnt.ensure(nt);
+    ws.ex_entries.ensure(nv * top_k);
+    ws.counters.ensure(64);
+    ws.gthr.ensure(nq);
+    ZB_CUDA(cudaMemsetAsync(ws.counters.p, 0, 64 * 4, s));
+    ZB_CUDA(cudaMemsetAsync(ws.gthr.p, 0xFF, (size_t)nq * 8, s));
+    ex_visits_kernel<<<(u32)((nv + 1 + 255) / 256), 256, 0, s>>>(nranges, nq, ntq, range_rows, n, top_k, ws.pj_off.p, ws.leaf_count.p,
+                                                                ws.ex_leaf.p, ws.ex_np.p, ws.ex_q.p, ws.order.p, ws.ex_ent_off.p,
+                                                                ws.ex_woff.p, ws.tile_leaf.p, ws.tile_first.p, ws.tile_cnt.p,
+                                                                ws.counters.p);
+    ZB_CUDA(cudaGetLastError());
+    ForestView f = store;
+    f.leaf_off = ws.pj_off.p;
+    f.leaf_len = ws.leaf_count.p;
+    f.num_trees = 1;
+    BucketMajor b = bm;
+    const double* q_rinv = nullptr;
+    if (metric == 0) {
+        ws.ex_q_rinv.ensure(nq);
+        launch_rinv(d_q, nq, f.dimp, ws.ex_q_rinv.p, s);
+        q_rinv = ws.ex_q_rinv.p;
+    }
+    ws.l2_filter = l2_filter && (metric == 1 || metric == 2) && bm.n2;
+    if (ws.l2_filter) {   // the filter's error bound per range
+        ws.ex_n2max.ensure(nranges);
+        launch_leaf_n2max(nranges, ws.pj_off.p, ws.leaf_count.p, bm.n2, ws.ex_n2max.p, s);
+        b.leaf_n2max = ws.ex_n2max.p;
+    }
+    t3_launch(ws, f, b, metric, d_q, q_rinv, nq, (u32)nv, ws.ex_leaf.p, ws.ex_np.p, ws.ex_q.p, ws.ex_ent_off.p, ws.ex_entries.p, top_k, kr,
+              nst, qcap, sms, ws.counters.p + 2, ws.counters.p + 3, s);
+    launch_merge_queries(nq, 1, ws.ex_woff.p, ws.ex_ent_off.p, ws.ex_entries.p, top_k, out_ord, out_bits, out_counts, s);
 }
 
 // =====================================================================================================

@@ -17,7 +17,13 @@ struct ScanWorkspace {
     bool filtered = false;
     int long_list_warps = 8;     // in: math warps per team for n' > 32 (knob long_list_warps: 8 = default, 4 = the short-list shape)
     cudaEvent_t ev2 = nullptr;   // after the second pass
-    DBuf<long long> pj_off;   // project3: first row of every row range
+    DBuf<long long> pj_off;   // project3 / exact_scan3: first row of every row range
+    // exact_scan3: visits (query-major: v = q * nranges + r), entry offsets, per-query visit offsets, the ranges' usable |row|^2
+    // maximum, the visits' lists and the queries' reciprocal norms
+    DBuf<u32> ex_leaf, ex_np, ex_q, ex_ent_off, ex_woff;
+    DBuf<float> ex_n2max;
+    DBuf<Entry> ex_entries;
+    DBuf<double> ex_q_rinv;
     DBuf<u8> tmp, sort_tmp;
     DBuf<u32> sort_key[2], sort_val[2];   // tile order: leaves sorted by cost
     bool launched = false;
@@ -70,6 +76,21 @@ void tile_scan3(ScanWorkspace& ws, const ForestView& f, const BucketMajor& bm, u
 bool project3_supported(int dimp);
 void project3(ScanWorkspace& ws, const float* d_rows, u64 n, const float* d_coef, const float* d_cst, int H, int dimp, u8* d_sign, int Hp,
               cudaStream_t s);
+// Exact mode of the third-generation scan (zb_index_search_exact): a plain [n][dimp] store (rows, ord, tomb of `store`, bm.rinv
+// / bm.n2 per row) cut into ranges of `range_rows` rows; every (range, query) pair is a visit with n' = top_k, the query tiles
+// of one range are handed out back to back so that they meet the range's rows in L2.  The visits' lists are merged into the
+// per-query top_k (out_*: [nq][top_k] / [nq]).  n = 0 gives empty lists.  l2_filter: L2 / L2 squared with top_k <= 16 go
+// through the dot-product filter and its exact second pass.
+#define ZB_EXACT_MAX_K 128   // the fused kernel's longest list
+struct ExactPlan {
+    u32 range_rows = 0;   // rows per range (a multiple of the 64-row stage)
+    u64 chunk = 0;        // queries per exact_scan3 call
+};
+// Range length and query chunk for n rows (the largest row count over all shards) and a batch of nq queries: enough tiles for
+// every team, visit arrays + entries + candidate lists + per_query_bytes x chunk within budget_bytes (at least one query).
+ExactPlan exact_plan(u64 n, u64 nq, int dimp, u32 top_k, bool l2_filter, u64 per_query_bytes, u64 budget_bytes);
+void exact_scan3(ScanWorkspace& ws, const ForestView& store, const BucketMajor& bm, u64 n, u32 metric, const float* d_q, u32 nq,
+                 u32 range_rows, u32 top_k, bool l2_filter, u64* out_ord, u64* out_bits, u32* out_counts, cudaStream_t s);
 void tile_scan_stats(ScanWorkspace& ws, cudaStream_t s, u64* tile_visits, u64* tile_pairs, u64* moved_bytes, float* kernel_ms,
                      u32* tiles, u64* unique_bytes, u64* flagged_visits = nullptr, u64* refined_rows = nullptr, float* refine_ms = nullptr);
 

@@ -194,6 +194,30 @@ class LSHIndex:
     def search_batch_device(self, nq: int, d_q_ptr: int, top_k: int, d_ord_ptr: int, d_bits_ptr: int, d_counts_ptr: int):
         _ffi.check(_ffi.lib().zb_index_search_batch_device(self._h, nq, d_q_ptr, top_k, d_ord_ptr, d_bits_ptr, d_counts_ptr))
 
+    # ---------------------------------------------------------------- exact (brute-force) search, zb_index_search_exact
+    def search_exact(self, query, top_k: int) -> List[Tuple[_uuid.UUID, int]]:
+        """The true top_k over every live row, ordered like `search` (ground truth for its recall)."""
+        ids, _, bits, counts = self.search_exact_batch(np.asarray(query, np.float32)[None, :], top_k)
+        c = int(counts[0])
+        return list(zip(_bytes_to_ids(ids[0, :c]), (int(b) for b in bits[0, :c])))
+
+    def search_exact_batch(self, queries, top_k: int, want_ids: bool = True):
+        """Returns (ids [nq,k,16] uint8 or None, ordinals [nq,k] uint64, distance bits [nq,k] uint64, counts [nq] uint32).
+        Sharded index: collective, every rank passes the same queries and gets the full results."""
+        q = np.ascontiguousarray(queries, dtype=np.float32).reshape(-1, self.dim)
+        nq = q.shape[0]
+        ids = np.empty((nq, top_k, 16), dtype=np.uint8) if want_ids else None
+        ords = np.empty((nq, top_k), dtype=np.uint64)
+        bits = np.empty((nq, top_k), dtype=np.uint64)
+        counts = np.zeros(nq, dtype=np.uint32)
+        _ffi.check(_ffi.lib().zb_index_search_exact(self._h, nq, q.ctypes.data, top_k,
+                                                    ids.ctypes.data if want_ids else None, ords.ctypes.data,
+                                                    bits.ctypes.data, counts.ctypes.data))
+        return ids, ords, bits, counts
+
+    def search_exact_batch_device(self, nq: int, d_q_ptr: int, top_k: int, d_ord_ptr: int, d_bits_ptr: int, d_counts_ptr: int):
+        _ffi.check(_ffi.lib().zb_index_search_exact_device(self._h, nq, d_q_ptr, top_k, d_ord_ptr, d_bits_ptr, d_counts_ptr))
+
     # ---- sharded index, scalable form: every rank passes (and gets back) only the slice of the batch it fronts ----
     def slice_bounds(self, nq_total: int, shard_rank: int, shard_count: int) -> Tuple[int, int]:
         """Queries [lo, hi) of a batch of nq_total that rank `shard_rank` of `shard_count` fronts (zb_index_search_slice)."""
@@ -371,6 +395,20 @@ class LSHIndex:
     def comm_init(self, unique_id: bytes) -> None:
         buf = (C.c_uint8 * 128).from_buffer_copy(unique_id)
         _ffi.check(_ffi.lib().zb_index_comm_init(self._h, buf))
+
+
+def recall_at_k(approx_ords, approx_counts, exact_ords, exact_counts) -> np.ndarray:
+    """Per query |approx ∩ exact| / count(exact) over the first counts[q] ordinals of each [nq, k] list; 1.0 where the
+    exact list is empty."""
+    a = np.asarray(approx_ords, dtype=np.uint64)
+    e = np.asarray(exact_ords, dtype=np.uint64)
+    ac = np.asarray(approx_counts).astype(np.int64).reshape(-1)
+    ec = np.asarray(exact_counts).astype(np.int64).reshape(-1)
+    out = np.ones(ec.shape[0], dtype=np.float64)
+    for q in range(ec.shape[0]):
+        if ec[q]:
+            out[q] = np.intersect1d(a[q, :ac[q]], e[q, :ec[q]]).size / ec[q]
+    return out
 
 
 def comm_unique_id() -> bytes:
