@@ -182,6 +182,35 @@ int zb_index_search_exact(zb_index* index, uint64_t nq, const float* queries, ui
 int zb_index_search_exact_device(zb_index* index, uint64_t nq, const float* d_queries, uint64_t top_k,
                                  uint64_t* d_out_ordinals, uint64_t* d_out_dist_bits, uint32_t* d_out_counts);
 
+/* Multi-probe search (this project's extension, DESIGN.md 3.9): raises recall without more trees by also visiting, in every
+ * tree, the leaves just across the query's closest hyperplanes.  probes = P, 0 <= P <= ZB_MAX_PROBES; P = 0 is exactly the
+ * plain call.  For P > 0, per query and tree:
+ *   1. tree_result runs unchanged (count cascade Q1, per-visit n' of Q2); its candidates are kept.
+ *   2. On the main path (the walk's first root-to-leaf descent) every inner node gets the margin key |v| / sqrt(n2), in f64
+ *      with IEEE round-to-nearest: v = (f64)dot(coef, q) + (f64)constant (the value point_is_above tests), n2 = (f64)
+ *      dot(coef, coef), both canonical f32 dots; key = +inf if v is NaN or n2 is 0 or not finite.
+ *   3. The min(P, path length) nodes with the smallest (key, depth) -- the shallower node first on equal keys -- are flipped:
+ *      from each one's other child the walk descends greedily (no further flips) to one probe leaf.  The probe leaves are
+ *      distinct from each other and from the main leaf.
+ *   4. A probe leaf with live rows contributes its min(live, top_k) nearest live rows, like a visit with n' = top_k; an empty
+ *      one contributes nothing and is not replaced.
+ *   5. The result is the top_k of the deduplicated union, in LSHIndex::search's order.
+ * The candidates of P + 1 include those of P, so recall never falls as P grows.  Every metric and scan path takes probes.
+ * zb_stats describes a probe batch like any other (last_visits / last_pairs include the probe visits).  Layout, 0xFF tail
+ * fill, NULL-able outputs, prefetch and sharding are those of the plain calls; on a sharded index every rank passes the same
+ * probes, as it passes the same top_k.  probes > ZB_MAX_PROBES returns ZB_ERR_INVALID. */
+#define ZB_MAX_PROBES 32
+int zb_index_search_probe(zb_index* index, uint64_t nq, const float* queries, uint64_t top_k, uint32_t probes, uint8_t* out_ids16,
+                          uint64_t* out_ordinals, uint64_t* out_dist_bits, uint32_t* out_counts);
+int zb_index_search_probe_device(zb_index* index, uint64_t nq, const float* d_queries, uint64_t top_k, uint32_t probes,
+                                 uint64_t* d_out_ordinals, uint64_t* d_out_dist_bits, uint32_t* d_out_counts);
+/* zb_index_search_slice / zb_index_search_slice_device with probes (collective on a sharded index). */
+int zb_index_search_slice_probe(zb_index* index, uint64_t nq_total, const float* slice_queries, uint64_t top_k, uint32_t probes,
+                                uint8_t* out_ids16, uint64_t* out_ordinals, uint64_t* out_dist_bits, uint32_t* out_counts);
+int zb_index_search_slice_probe_device(zb_index* index, uint64_t nq_total, const float* d_slice_queries, uint64_t top_k,
+                                       uint32_t probes, uint64_t* d_out_ordinals, uint64_t* d_out_dist_bits,
+                                       uint32_t* d_out_counts);
+
 /* Bucket keys: the root-to-leaf sign path of Hyperplane::point_is_above decisions (lsh.rs:39-43 along
  * :350-366), MSB = root, 1 = above/right, for every (row, tree): out_keys/out_depths/out_leaves are
  * [n][num_trees] (a path longer than 64 keeps its last 64 bits; out_leaves is the leaf number of

@@ -275,21 +275,28 @@ class LSHIndex {
     /// lsh.rs:506-529 (without quirk Q12: trees go too).
     void clear() const { check(zb_index_clear(raw())); }
 
-    /// lsh.rs:544-565 for ONE query -- prefer search_batch.
+    /// lsh.rs:544-565 for ONE query -- prefer search_batch.  probes > 0: multi-probe search (zb_index_search_probe,
+    /// DESIGN 3.9); 0 is the reference's search.
     template <class Met>
-    std::vector<std::pair<Uuid, DistanceUnit>> search(const Embedding<N>& query, size_t top_k, const Met& metric) const {
+    std::vector<std::pair<Uuid, DistanceUnit>> search(const Embedding<N>& query, size_t top_k, const Met& metric,
+                                                      uint32_t probes = 0) const {
         if (Met::ZB_METRIC != metric_ || metric.zb_power() != power_)
             throw Error(ZB_ERR_INVALID, "this device index was created for another metric");
-        return std::move(search_batch(std::vector<Embedding<N>>{query}, top_k)[0]);
+        return std::move(search_batch(std::vector<Embedding<N>>{query}, top_k, probes)[0]);
     }
     /// The whole batch in one device call (replaces the par_iter of core.rs:299-303): per query, ascending (distance
     /// bits, id), at most top_k entries.
-    std::vector<std::vector<std::pair<Uuid, DistanceUnit>>> search_batch(const std::vector<Embedding<N>>& queries, size_t top_k) const {
+    std::vector<std::vector<std::pair<Uuid, DistanceUnit>>> search_batch(const std::vector<Embedding<N>>& queries, size_t top_k,
+                                                                         uint32_t probes = 0) const {
         const size_t nq = queries.size();
         std::vector<uint8_t> ids(nq * top_k * 16 + 1);
         std::vector<uint64_t> bits(nq * top_k + 1);
         std::vector<uint32_t> counts(nq + 1, 0);
-        check(zb_index_search_batch(raw(), nq, nq ? queries[0].data() : nullptr, top_k, ids.data(), nullptr, bits.data(), counts.data()));
+        if (probes)
+            check(zb_index_search_probe(raw(), nq, nq ? queries[0].data() : nullptr, top_k, probes, ids.data(), nullptr, bits.data(),
+                                        counts.data()));
+        else
+            check(zb_index_search_batch(raw(), nq, nq ? queries[0].data() : nullptr, top_k, ids.data(), nullptr, bits.data(), counts.data()));
         std::vector<std::vector<std::pair<Uuid, DistanceUnit>>> out(nq);
         for (size_t q = 0; q < nq; ++q)
             for (uint32_t i = 0; i < counts[q]; ++i) {
@@ -644,10 +651,11 @@ class Database {
         return query_vectors(s_->model.embed_documents(documents), number_of_results);
     }
     /// core.rs:290-313: query index -> (document id -> document bytes).
-    std::map<size_t, std::map<Uuid, Bytes>> query_vectors(const std::vector<Embedding<N>>& vectors, size_t number_of_results) const {
+    std::map<size_t, std::map<Uuid, Bytes>> query_vectors(const std::vector<Embedding<N>>& vectors, size_t number_of_results,
+                                                          uint32_t probes = 0) const {
         std::map<size_t, std::map<Uuid, Bytes>> results;
         if (index.no_vectors()) return results;
-        auto all = index.search_batch(vectors, number_of_results);  // was: vectors.into_par_iter() ... index.search(x, ..)
+        auto all = index.search_batch(vectors, number_of_results, probes);  // was: vectors.into_par_iter() ... index.search(x, ..)
         for (size_t q = 0; q < all.size(); ++q) {
             std::map<Uuid, Bytes>& m = results[q];
             for (const auto& hit : all[q]) {

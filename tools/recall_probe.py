@@ -2,7 +2,8 @@
 
 Builds the index the way bench.py does (rows and queries from zb_synth_fill_device with the same seeds: rows seed S, queries
 seed S + 1), runs the LSH search (zb_index_search_batch_device) and the exact search (zb_index_search_exact_device) on the same
-queries and prints one JSON line per forest shape (--trees takes a list):
+queries and prints one JSON line per (forest shape, probes) (--trees and --probes take lists; probes > 0 runs the multi-probe
+search, zb_index_search_probe_device):
 
   recall@1, recall@k         mean over all queries of recall_at_k (the exact top-k is the ground truth)
   lsh_qps, exact_qps          host clock around device-resident calls that end in a synchronise, after warm-up
@@ -10,10 +11,13 @@ queries and prints one JSON line per forest shape (--trees takes a list):
   exact_bytes_one_pass_per_chunk / exact_bytes_no_reuse
                               algorithmic HBM bytes: the rows once per query chunk, and once per 16-query tile (no L2 reuse)
   lsh_tile_pairs_per_s        the LSH tile kernel's own rate (last_tile_pairs / last_ms_tile_kernel), same process
+  lsh_ms_plan / _scan / _total, plan_share
+                              the last LSH batch's phases (zb_stats) and the plan walk's share of its total
+  visits_per_query, pairs_per_query
   gpu, power_limit_w          read in the same call
   parity                      a few queries of the exact result against the oracle's brute force (bits and ordinals)
 
-  python tools/recall_probe.py --trees 1,4,8 --kind 1 --out profiles/r03_recall_config2_clustered.jsonl
+  python tools/recall_probe.py --trees 1,4,8 --probes 0,1,2,4,8 --kind 1 --queries-from held-out --out profiles/x.jsonl
 Under torchrun every rank builds its shard (add_owned_device) and both searches run sharded (the exact one is collective).
 """
 from __future__ import annotations
@@ -74,6 +78,7 @@ def main():
     ap.add_argument("--metric", default="l2", choices=list(METRICS))
     ap.add_argument("--max-node-size", type=int, default=2048)
     ap.add_argument("--trees", default="4", help="comma-separated list: one index per value")
+    ap.add_argument("--probes", default="0", help="comma-separated list: one LSH measurement per value and forest")
     ap.add_argument("--kind", type=int, default=1, help="synthetic rows: 0 uniform in [-1, 1), 1 clustered (bench.py's)")
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--queries-from", default="bench", choices=["bench", "held-out"],
@@ -119,37 +124,47 @@ def main():
         torch.cuda.empty_cache()
 
         args = (nq, d_q.data_ptr(), k, d_ord.data_ptr(), d_bits.data_ptr(), d_cnt.data_ptr())
-        lsh = lambda: ix.search_batch_device(*args)  # noqa: E731
         exact = lambda: ix.search_exact_batch_device(*args)  # noqa: E731
         for _ in range(a.warmup):
-            lsh()
             exact()
-        t_lsh = timed(lsh, a.reps)
-        st = ix.stats()
-        a_ord, a_cnt = d_ord.cpu().numpy().view(np.uint64).copy(), d_cnt.cpu().numpy().copy()
+        st_before = ix.stats()
         t_exact = timed(exact, a.reps)
         e_ord, e_bits, e_cnt = d_ord.cpu().numpy().view(np.uint64).copy(), d_bits.cpu().numpy().view(np.uint64).copy(), d_cnt.cpu().numpy().copy()
         st_after = ix.stats()
-        rec_k = z.recall_at_k(a_ord, a_cnt, e_ord, e_cnt)
-        rec_1 = z.recall_at_k(a_ord[:, :1], np.minimum(a_cnt, 1), e_ord[:, :1], np.minimum(e_cnt, 1))
         dimp = -(-a.dim // 16) * 16
         filt = a.metric != "cosine" and k <= 16 and dimp >= 128
         chunks, range_rows = exact_chunks(n if G == 1 else -(-n // G), nq, k, dimp, filt)
         row_bytes = n * dimp * 4
-        line = {
-            "rows": n, "dim": a.dim, "metric": a.metric, "kind": "clustered" if a.kind == 1 else "uniform", "queries_from": a.queries_from, "trees": trees,
-            "max_node_size": a.max_node_size, "queries": nq, "topk": k, "gpus": G, "gpu": name, "power_limit_w": power,
-            "recall_at_1": float(rec_1.mean()), f"recall_at_{k}": float(rec_k.mean()), "recall_at_k_min": float(rec_k.min()),
-            "lsh_s": t_lsh, "lsh_qps": nq / t_lsh, "exact_s": t_exact, "exact_qps": nq / t_exact,
-            "exact_pairs_per_s": n * nq / t_exact,
-            "lsh_tile_pairs_per_s": st["last_tile_pairs"] / (st["last_ms_tile_kernel"] * 1e-3) if st["last_ms_tile_kernel"] else None,
-            "lsh_pairs": st["last_pairs"], "lsh_ms_tile_kernel": st["last_ms_tile_kernel"],
-            "exact_query_chunks": chunks, "exact_range_rows": range_rows, "exact_l2_filter": filt,
-            "exact_bytes_one_pass_per_chunk": row_bytes * chunks, "exact_bytes_no_reuse": row_bytes * -(-nq // 16),
-            "exact_bytes_per_s_one_pass_per_chunk": row_bytes * chunks / t_exact,
-            "stats_untouched_by_exact": {kk: st[kk] for kk in st if kk.startswith("last_")} ==
-                                        {kk: st_after[kk] for kk in st_after if kk.startswith("last_")},
-        }
+        lines = []
+        for probes in (int(p) for p in a.probes.split(",")):
+            lsh = lambda: ix.search_batch_device(*args, probes=probes)  # noqa: E731
+            for _ in range(a.warmup):
+                lsh()
+            t_lsh = timed(lsh, a.reps)
+            st = ix.stats()
+            a_ord, a_cnt = d_ord.cpu().numpy().view(np.uint64).copy(), d_cnt.cpu().numpy().copy()
+            rec_k = z.recall_at_k(a_ord, a_cnt, e_ord, e_cnt)
+            rec_1 = z.recall_at_k(a_ord[:, :1], np.minimum(a_cnt, 1), e_ord[:, :1], np.minimum(e_cnt, 1))
+            line = {
+                "rows": n, "dim": a.dim, "metric": a.metric, "kind": "clustered" if a.kind == 1 else "uniform", "queries_from": a.queries_from,
+                "trees": trees, "probes": probes, "max_node_size": a.max_node_size, "queries": nq, "topk": k, "gpus": G, "gpu": name,
+                "power_limit_w": power,
+                "recall_at_1": float(rec_1.mean()), f"recall_at_{k}": float(rec_k.mean()), "recall_at_k_min": float(rec_k.min()),
+                "lsh_s": t_lsh, "lsh_qps": nq / t_lsh, "exact_s": t_exact, "exact_qps": nq / t_exact,
+                "exact_pairs_per_s": n * nq / t_exact,
+                "lsh_tile_pairs_per_s": st["last_tile_pairs"] / (st["last_ms_tile_kernel"] * 1e-3) if st["last_ms_tile_kernel"] else None,
+                "lsh_pairs": st["last_pairs"], "lsh_ms_tile_kernel": st["last_ms_tile_kernel"],
+                "lsh_ms_plan": st["last_ms_plan"], "lsh_ms_scan": st["last_ms_scan"], "lsh_ms_total": st["last_ms_total"],
+                "plan_share": st["last_ms_plan"] / st["last_ms_total"] if st["last_ms_total"] else None,
+                "visits_per_query": st["last_visits"] / nq, "pairs_per_query": st["last_pairs"] / nq,
+                "exact_query_chunks": chunks, "exact_range_rows": range_rows, "exact_l2_filter": filt,
+                "exact_bytes_one_pass_per_chunk": row_bytes * chunks, "exact_bytes_no_reuse": row_bytes * -(-nq // 16),
+                "exact_bytes_per_s_one_pass_per_chunk": row_bytes * chunks / t_exact,
+                "stats_untouched_by_exact": {kk: st_before[kk] for kk in st_before if kk.startswith("last_")} ==
+                                            {kk: st_after[kk] for kk in st_after if kk.startswith("last_")},
+            }
+            lines.append(line)
+        line = lines[0]
         if a.parity and rank == 0:
             rows = zo.synth(0, 1, n, a.dim, a.seed, a.kind)
             qs = zo.synth(q_first, 1, a.parity, a.dim, q_seed, a.kind)
@@ -162,11 +177,12 @@ def main():
             line["parity"] = {"queries": a.parity, "bit_exact": ok}
             del rows
         if rank == 0:
-            s = json.dumps(line)
-            print(s, flush=True)
-            if a.out:
-                with open(a.out, "a") as f:
-                    f.write(s + "\n")
+            for ln in lines:
+                s = json.dumps(ln)
+                print(s, flush=True)
+                if a.out:
+                    with open(a.out, "a") as f:
+                        f.write(s + "\n")
         ix.close()
     if world > 1:
         dist.destroy_process_group()

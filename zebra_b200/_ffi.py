@@ -114,6 +114,10 @@ SYMBOLS = {
     "zb_index_search_prefetch": (C.c_int, [_vp, _u64, _vp]),
     "zb_index_search_exact": (C.c_int, [_vp, _u64, _vp, _u64, _vp, _vp, _vp, _vp]),
     "zb_index_search_exact_device": (C.c_int, [_vp, _u64, _vp, _u64, _vp, _vp, _vp]),
+    "zb_index_search_probe": (C.c_int, [_vp, _u64, _vp, _u64, C.c_uint32, _vp, _vp, _vp, _vp]),
+    "zb_index_search_probe_device": (C.c_int, [_vp, _u64, _vp, _u64, C.c_uint32, _vp, _vp, _vp]),
+    "zb_index_search_slice_probe": (C.c_int, [_vp, _u64, _vp, _u64, C.c_uint32, _vp, _vp, _vp, _vp]),
+    "zb_index_search_slice_probe_device": (C.c_int, [_vp, _u64, _vp, _u64, C.c_uint32, _vp, _vp, _vp]),
     "zb_index_hash": (C.c_int, [_vp, _u64, _vp, _vp, _vp, _vp]),
     "zb_index_hash_device": (C.c_int, [_vp, _u64, _vp, _vp, _vp, _vp]),
     "zb_index_forest_sizes": (C.c_int, [_vp, _vp]),

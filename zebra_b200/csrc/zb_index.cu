@@ -997,7 +997,8 @@ namespace zb {
 // all nq results (on every rank).  Sharded with sliced == true (the scalable form): d_q holds only the slice this rank
 // fronts, queries [rank * nqp, (rank + 1) * nqp) with nqp = ceil(nq / G); the slices are allgathered over NVLink into
 // q_all, and the outputs receive the results of the rank's own slice only (no result allgather).
-static void search_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64* d_out_ord, u64* d_out_bits,
+// probes > 0: multi-probe walk (DESIGN 3.9); the visits it appends go through the same compaction, scan and merge.
+static void search_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u32 probes, u64* d_out_ord, u64* d_out_bits,
                           u32* d_out_counts, bool sliced) {
     cudaStream_t s = ix->stream;
     const u32 T = ix->T;
@@ -1071,7 +1072,9 @@ static void search_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64
     const bool gen3 = ix->p_scan_gen != 2 && tile_scan3_supported(ix->dimp, (u32)top_k);
     const bool tile_on = ix->opt.metric <= ZB_METRIC_L2 && ix->p_use_tile_scan && ix->opt.max_node_size >= (u64)ix->p_tile_min_rows &&
                          (gen3 || tile_scan_supported(ix->dimp, (u32)top_k)) && ix->ensure_bucket_major();
-    u64 v_cap = std::max<u64>(ix->v_leaf.cap ? ix->v_leaf.cap - 1 : 0, nw + nw / 2 + 1024);
+    u64 v_cap = std::max<u64>(ix->v_leaf.cap ? ix->v_leaf.cap - 1 : 0, nw * (1 + (u64)probes) + nw / 2 + 1024);
+    // a walker's region holds its cascade (31 visits by default) plus its probe visits, so the first probe batch needs no replan
+    if (probes) ix->vpw = std::max<u32>(ix->vpw, 32 + probes);
     if (sharded && !ix->x_cap) ix->x_cap = (u32)std::min<u64>(nwl + nwl / 2 + 64, 0x7FFFFFFFull);
     ix->plan_totals.ensure(8);
     // Three nested retries, each decided from data every rank sees identically or from purely local state:
@@ -1102,7 +1105,7 @@ static void search_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64
                 ix->w_tail.ensure(nwl + 2);
                 tail = ix->w_tail.p;
             }
-            launch_plan(f, d_q_mine, (u32)qn, (u32)top_k, ix->vpw, ix->w_visits.p, ix->w_counts.p, ix->w_flag.p, tail, s);
+            launch_plan(f, d_q_mine, (u32)qn, (u32)top_k, probes, ix->vpw, ix->w_visits.p, ix->w_counts.p, ix->w_flag.p, tail, s);
             if (tail) ix->st.last_total_launches += 1;
             ix->trace_mark("plan walk");
             if (sharded) {
@@ -1814,7 +1817,7 @@ int zb_index_no_trees(zb_index* ix, int* out) {
 
 // Batches beyond 131072 queries are cut into chunks (walker count < 2^31, bounded workspaces).  sliced: see search_device;
 // the chunks of a sliced call are chunks of the whole batch, so every rank sees the same sequence of collectives.
-static void search_entry_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64* d_out_ord, u64* d_out_bits,
+static void search_entry_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u32 probes, u64* d_out_ord, u64* d_out_bits,
                                 u32* d_out_counts, bool sliced, bool exact = false) {
     ix->use_device();
     const u64 G = ix->G;
@@ -1830,7 +1833,7 @@ static void search_entry_device(zb_index* ix, u64 nq, const float* d_q, u64 top_
         }
         const float* q = stage_queries_device(ix, d_q + in_off * (u64)ix->dim, mine);
         if (exact) exact_device(ix, c, q, top_k, d_out_ord + in_off * top_k, d_out_bits + in_off * top_k, d_out_counts + in_off);
-        else search_device(ix, c, q, top_k, d_out_ord + in_off * top_k, d_out_bits + in_off * top_k, d_out_counts + in_off, sliced);
+        else search_device(ix, c, q, top_k, probes, d_out_ord + in_off * top_k, d_out_bits + in_off * top_k, d_out_counts + in_off, sliced);
         in_off += mine;
     }
     ix->sync();
@@ -1842,7 +1845,7 @@ int zb_index_search_batch_device(zb_index* ix, uint64_t nq, const float* d_q, ui
     ZB_REQUIRE(ix && (d_q || !nq) && ((d_out_ord && d_out_bits && d_out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
     ZB_REQUIRE(top_k <= ZB_MAX_TOPK, ZB_ERR_INVALID, "top_k %llu exceeds %d", (unsigned long long)top_k, ZB_MAX_TOPK);
     std::lock_guard<std::mutex> lk(ix->mu);
-    search_entry_device(ix, nq, d_q, top_k, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, false);
+    search_entry_device(ix, nq, d_q, top_k, 0, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, false);
     ZB_API_END
 }
 int zb_index_search_slice_device(zb_index* ix, uint64_t nq_total, const float* d_q, uint64_t top_k, uint64_t* d_out_ord,
@@ -1851,13 +1854,13 @@ int zb_index_search_slice_device(zb_index* ix, uint64_t nq_total, const float* d
     ZB_REQUIRE(ix, ZB_ERR_INVALID, "NULL argument");
     ZB_REQUIRE(top_k <= ZB_MAX_TOPK, ZB_ERR_INVALID, "top_k %llu exceeds %d", (unsigned long long)top_k, ZB_MAX_TOPK);
     std::lock_guard<std::mutex> lk(ix->mu);
-    search_entry_device(ix, nq_total, d_q, top_k, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, true);
+    search_entry_device(ix, nq_total, d_q, top_k, 0, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, true);
     ZB_API_END
 }
 
 // Host buffers in, host buffers out.  sliced: `queries` and the outputs hold this rank's slices only.
-static void search_entry_host(zb_index* ix, u64 nq, const float* queries, u64 top_k, uint8_t* out_ids16, u64* out_ordinals,
-                              u64* out_bits, u32* out_counts, bool sliced, bool exact = false) {
+static void search_entry_host(zb_index* ix, u64 nq, const float* queries, u64 top_k, u32 probes, uint8_t* out_ids16,
+                              u64* out_ordinals, u64* out_bits, u32* out_counts, bool sliced, bool exact = false) {
     ix->use_device();
     cudaStream_t s = ix->stream;
     const u64 G = ix->G;
@@ -1898,7 +1901,7 @@ static void search_entry_host(zb_index* ix, u64 nq, const float* queries, u64 to
         ix->o_bits.ensure(mine * top_k + 1);
         ix->o_counts2.ensure(mine + 1);
         if (exact) exact_device(ix, c, ix->q_stage.p, top_k, ix->o_ord.p, ix->o_bits.p, ix->o_counts2.p);
-        else search_device(ix, c, ix->q_stage.p, top_k, ix->o_ord.p, ix->o_bits.p, ix->o_counts2.p, sliced);
+        else search_device(ix, c, ix->q_stage.p, top_k, probes, ix->o_ord.p, ix->o_bits.p, ix->o_counts2.p, sliced);
         if (!out_ordinals && out_ids16) ord_tmp.resize(mine * top_k);
         u64* ords = out_ordinals ? out_ordinals + in_off * top_k : ord_tmp.data();
         if (top_k && mine) {
@@ -1924,7 +1927,7 @@ int zb_index_search_batch(zb_index* ix, uint64_t nq, const float* queries, uint6
     ZB_REQUIRE(ix && (queries || !nq) && ((out_bits && out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
     ZB_REQUIRE(top_k <= ZB_MAX_TOPK, ZB_ERR_INVALID, "top_k %llu exceeds %d", (unsigned long long)top_k, ZB_MAX_TOPK);
     std::lock_guard<std::mutex> lk(ix->mu);
-    search_entry_host(ix, nq, queries, top_k, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, false);
+    search_entry_host(ix, nq, queries, top_k, 0, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, false);
     ZB_API_END
 }
 static void exact_check(zb_index* ix, u64 top_k) {
@@ -1943,7 +1946,7 @@ int zb_index_search_exact(zb_index* ix, uint64_t nq, const float* queries, uint6
     ZB_REQUIRE(ix && (queries || !nq) && ((out_bits && out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
     std::lock_guard<std::mutex> lk(ix->mu);
     exact_check(ix, top_k);
-    search_entry_host(ix, nq, queries, top_k, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, false, true);
+    search_entry_host(ix, nq, queries, top_k, 0, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, false, true);
     ZB_API_END
 }
 int zb_index_search_exact_device(zb_index* ix, uint64_t nq, const float* d_q, uint64_t top_k, uint64_t* d_out_ord,
@@ -1952,7 +1955,7 @@ int zb_index_search_exact_device(zb_index* ix, uint64_t nq, const float* d_q, ui
     ZB_REQUIRE(ix && (d_q || !nq) && ((d_out_ord && d_out_bits && d_out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
     std::lock_guard<std::mutex> lk(ix->mu);
     exact_check(ix, top_k);
-    search_entry_device(ix, nq, d_q, top_k, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, false, true);
+    search_entry_device(ix, nq, d_q, top_k, 0, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, false, true);
     ZB_API_END
 }
 int zb_index_search_prefetch(zb_index* ix, uint64_t n, const float* queries) {
@@ -1996,7 +1999,49 @@ int zb_index_search_slice(zb_index* ix, uint64_t nq_total, const float* queries,
     ZB_REQUIRE(ix, ZB_ERR_INVALID, "NULL argument");
     ZB_REQUIRE(top_k <= ZB_MAX_TOPK, ZB_ERR_INVALID, "top_k %llu exceeds %d", (unsigned long long)top_k, ZB_MAX_TOPK);
     std::lock_guard<std::mutex> lk(ix->mu);
-    search_entry_host(ix, nq_total, queries, top_k, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, true);
+    search_entry_host(ix, nq_total, queries, top_k, 0, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, true);
+    ZB_API_END
+}
+
+// Multi-probe forms of the four search calls (DESIGN 3.9); probes = 0 is the plain call.
+static void probe_check(u64 top_k, u32 probes) {
+    ZB_REQUIRE(top_k <= ZB_MAX_TOPK, ZB_ERR_INVALID, "top_k %llu exceeds %d", (unsigned long long)top_k, ZB_MAX_TOPK);
+    ZB_REQUIRE(probes <= ZB_MAX_PROBES, ZB_ERR_INVALID, "probes %u exceeds %d", probes, ZB_MAX_PROBES);
+}
+int zb_index_search_probe(zb_index* ix, uint64_t nq, const float* queries, uint64_t top_k, uint32_t probes, uint8_t* out_ids16,
+                          uint64_t* out_ordinals, uint64_t* out_bits, uint32_t* out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && (queries || !nq) && ((out_bits && out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
+    probe_check(top_k, probes);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    search_entry_host(ix, nq, queries, top_k, probes, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, false);
+    ZB_API_END
+}
+int zb_index_search_probe_device(zb_index* ix, uint64_t nq, const float* d_q, uint64_t top_k, uint32_t probes, uint64_t* d_out_ord,
+                                 uint64_t* d_out_bits, uint32_t* d_out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && (d_q || !nq) && ((d_out_ord && d_out_bits && d_out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
+    probe_check(top_k, probes);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    search_entry_device(ix, nq, d_q, top_k, probes, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, false);
+    ZB_API_END
+}
+int zb_index_search_slice_probe(zb_index* ix, uint64_t nq_total, const float* queries, uint64_t top_k, uint32_t probes,
+                                uint8_t* out_ids16, uint64_t* out_ordinals, uint64_t* out_bits, uint32_t* out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix, ZB_ERR_INVALID, "NULL argument");
+    probe_check(top_k, probes);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    search_entry_host(ix, nq_total, queries, top_k, probes, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, true);
+    ZB_API_END
+}
+int zb_index_search_slice_probe_device(zb_index* ix, uint64_t nq_total, const float* d_q, uint64_t top_k, uint32_t probes,
+                                       uint64_t* d_out_ord, uint64_t* d_out_bits, uint32_t* d_out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix, ZB_ERR_INVALID, "NULL argument");
+    probe_check(top_k, probes);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    search_entry_device(ix, nq_total, d_q, top_k, probes, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, true);
     ZB_API_END
 }
 

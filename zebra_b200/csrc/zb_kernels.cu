@@ -23,9 +23,13 @@ namespace zb {
 // first FFMA then stalls with 4-6 requests in flight), so the requests are `volatile` loads (kept in program order; they
 // bypass L1, which holds nothing of a deep node's plane anyway) and the head of every accumulator chain is made to depend
 // on the LAST request by or-ing in `bits & zero`.  Same fused multiply-add sequence per accumulator lane as quad_dot.
+// N2 (probe walk, first descent): the plane's canonical self-dot is accumulated from the same loads into *n2.
+template <bool N2 = false>
 __device__ __forceinline__ float quad_dot_tail(const float4* __restrict__ a, const float4* __restrict__ b, int chunks, int sub, unsigned mask,
-                                               const u32 zero /* 0, derived from a kernel argument: the compiler cannot know */) {
+                                               const u32 zero /* 0, derived from a kernel argument: the compiler cannot know */,
+                                               float* n2 = nullptr) {
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 acc2 = make_float4(0.f, 0.f, 0.f, 0.f);
     int c = 0;
     for (; c + 24 <= chunks; c += 24) {
         float4 av[24];
@@ -38,7 +42,10 @@ __device__ __forceinline__ float quad_dot_tail(const float4* __restrict__ a, con
         av[0].z = __uint_as_float(__float_as_uint(av[0].z) | dep);
         av[0].w = __uint_as_float(__float_as_uint(av[0].w) | dep);
 #pragma unroll
-        for (int i = 0; i < 24; ++i) fma4(acc, av[i], __ldg(b + (c + i) * 4 + sub));   // the query: L1 hits
+        for (int i = 0; i < 24; ++i) {
+            fma4(acc, av[i], __ldg(b + (c + i) * 4 + sub));   // the query: L1 hits
+            if (N2) fma4(acc2, av[i], av[i]);
+        }
     }
     for (; c + 4 <= chunks; c += 4) {
         float4 a0 = __ldg(a + (c + 0) * 4 + sub), a1 = __ldg(a + (c + 1) * 4 + sub);
@@ -49,25 +56,79 @@ __device__ __forceinline__ float quad_dot_tail(const float4* __restrict__ a, con
         fma4(acc, a1, b1);
         fma4(acc, a2, b2);
         fma4(acc, a3, b3);
+        if (N2) {
+            fma4(acc2, a0, a0);
+            fma4(acc2, a1, a1);
+            fma4(acc2, a2, a2);
+            fma4(acc2, a3, a3);
+        }
     }
-    for (; c < chunks; ++c) fma4(acc, __ldg(a + c * 4 + sub), __ldg(b + c * 4 + sub));
+    for (; c < chunks; ++c) {
+        const float4 ac = __ldg(a + c * 4 + sub);
+        fma4(acc, ac, __ldg(b + c * 4 + sub));
+        if (N2) fma4(acc2, ac, ac);
+    }
+    if (N2) *n2 = quad_reduce16(acc2, mask);
     return quad_reduce16(acc, mask);
+}
+
+// quad_dot (zb_device.cuh) with the plane's canonical self-dot accumulated from the same loads into n2.
+__device__ __forceinline__ float quad_dot_n2(const float4* __restrict__ a, const float4* __restrict__ b, int chunks, int sub,
+                                             unsigned mask, float& n2) {
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f), acc2 = make_float4(0.f, 0.f, 0.f, 0.f);
+    int c = 0;
+    for (; c + 4 <= chunks; c += 4) {
+        float4 a0 = __ldg(a + (c + 0) * 4 + sub), a1 = __ldg(a + (c + 1) * 4 + sub);
+        float4 a2 = __ldg(a + (c + 2) * 4 + sub), a3 = __ldg(a + (c + 3) * 4 + sub);
+        float4 b0 = __ldg(b + (c + 0) * 4 + sub), b1 = __ldg(b + (c + 1) * 4 + sub);
+        float4 b2 = __ldg(b + (c + 2) * 4 + sub), b3 = __ldg(b + (c + 3) * 4 + sub);
+        fma4(acc, a0, b0);
+        fma4(acc, a1, b1);
+        fma4(acc, a2, b2);
+        fma4(acc, a3, b3);
+        fma4(acc2, a0, a0);
+        fma4(acc2, a1, a1);
+        fma4(acc2, a2, a2);
+        fma4(acc2, a3, a3);
+    }
+    for (; c < chunks; ++c) {
+        const float4 ac = __ldg(a + c * 4 + sub);
+        fma4(acc, ac, __ldg(b + c * 4 + sub));
+        fma4(acc2, ac, ac);
+    }
+    n2 = quad_reduce16(acc2, mask);
+    return quad_reduce16(acc, mask);
+}
+
+// Margin key of a main-path node (DESIGN 3.9): |v| / sqrt(n2) in f64, v = (f64)dot + (f64)cst the value point_is_above tests,
+// n2 the plane's canonical self-dot; +inf when v is NaN or n2 is 0 or not finite.
+__device__ __forceinline__ double probe_key(float dot, float cst, float n2f) {
+    const double v = __dadd_rn((double)dot, (double)cst);
+    const double n2 = (double)n2f;
+    if (isnan(v) || !(n2 > 0.0) || isinf(n2)) return __longlong_as_double(0x7FF0000000000000ll);
+    return __ddiv_rn(fabs(v), __dsqrt_rn(n2));
 }
 
 // One walker.  TAIL == false (plan_walk_kernel): with `defer` set, a walker whose first leaf cannot fill its budget (the count
 // cascade goes on) is put on the tail list and left to plan_walk_tail_kernel, which walks it again from the root with
 // quad_dot_tail; returns without writing anything for it.
-template <bool TAIL>
+// PROBE (multi-probe search, DESIGN 3.9): the first descent also keeps each main-path node's margin key and backup child; after
+// the reference walk the `probes` nodes with the smallest (key, depth) are flipped, each backup side is descended greedily to
+// one probe leaf, and every probe leaf with live rows is appended as a visit with n' = top_k.
+template <bool TAIL, bool PROBE = false>
 __device__ __forceinline__ void plan_walk_one(const ForestView& f, const float* __restrict__ queries, const u32 w, const int sub,
                                               const unsigned mask, const u32 top_k, const u32 vpw, uint2* __restrict__ wvisits,
                                               u32* __restrict__ wcounts, u32* __restrict__ overflow, u32* __restrict__ tail_list,
-                                              u32* __restrict__ tail_count) {
+                                              u32* __restrict__ tail_count, const u32 probes = 0) {
     const u32 q = w / (u32)f.num_trees;
     const u32 t = w - q * (u32)f.num_trees;
     const float4* qv = reinterpret_cast<const float4*>(queries + (size_t)q * f.dimp);
 
     int stack_node[ZB_MAX_DEPTH + 2];
     int stack_n[ZB_MAX_DEPTH + 2];
+    double pkey[PROBE ? ZB_MAX_DEPTH + 2 : 1];  // main path: margin key by depth
+    int pback[PROBE ? ZB_MAX_DEPTH + 2 : 1];    // main path: backup child by depth
+    int plen = -1;                              // main-path length, known once the first descent has reached its leaf
     int sp = 0;
     int cur = f.roots[t];
     int n = (int)top_k;
@@ -78,16 +139,25 @@ __device__ __forceinline__ void plan_walk_one(const ForestView& f, const float* 
         while (nd.x >= 0) {  // inner node: lsh.rs:333-338
             const float cst = f.cst[nd.x];
             const float4* plane = reinterpret_cast<const float4*>(f.coef + (size_t)nd.x * f.dimp);
-            float d = TAIL ? quad_dot_tail(plane, qv, f.chunks, sub, mask, top_k >> 31) : quad_dot(plane, qv, f.chunks, sub, mask);
+            float d, n2 = 0.f;
+            if (PROBE && plen < 0)
+                d = TAIL ? quad_dot_tail<true>(plane, qv, f.chunks, sub, mask, top_k >> 31, &n2) : quad_dot_n2(plane, qv, f.chunks, sub, mask, n2);
+            else
+                d = TAIL ? quad_dot_tail(plane, qv, f.chunks, sub, mask, top_k >> 31) : quad_dot(plane, qv, f.chunks, sub, mask);
             bool ab = above_from_dot(d, cst);
             if (sp < ZB_MAX_DEPTH + 2) {
                 stack_node[sp] = ab ? nd.y : nd.z;  // backup
                 stack_n[sp] = n;
+                if (PROBE && plen < 0) {
+                    pkey[sp] = probe_key(d, cst, n2);
+                    pback[sp] = ab ? nd.y : nd.z;
+                }
             }
             ++sp;
             cur = ab ? nd.z : nd.y;  // main
             nd = f.nodes[cur];
         }
+        if (PROBE && plen < 0) plen = sp;
         if (sp > ZB_MAX_DEPTH + 2) {  // cannot happen for forests accepted by the host (depth checked)
             ovf = 2;
             break;
@@ -115,6 +185,35 @@ __device__ __forceinline__ void plan_walk_one(const ForestView& f, const float* 
             }
         }
         if (!again) break;
+    }
+    if (PROBE && !ovf) {
+        // the i-th probe is the smallest (key, depth) after the (i-1)-th: depths are distinct, so no node is picked twice
+        const int np = (int)probes < plen ? (int)probes : plen;
+        double lk = -1.0;
+        int ld = -1;
+        for (int i = 0; i < np; ++i) {
+            double bk = __longlong_as_double(0x7FF0000000000000ll);
+            int bd = 0x7FFFFFFF;
+            for (int dd = 0; dd < plen; ++dd) {
+                const double k = pkey[dd];
+                if ((k > lk || (k == lk && dd > ld)) && (k < bk || (k == bk && dd < bd))) {
+                    bk = k;
+                    bd = dd;
+                }
+            }
+            lk = bk;
+            ld = bd;
+            int4 nd = f.nodes[pback[bd]];
+            while (nd.x >= 0) {  // greedy descent of the backup side, no further flips
+                const float4* plane = reinterpret_cast<const float4*>(f.coef + (size_t)nd.x * f.dimp);
+                float d = TAIL ? quad_dot_tail(plane, qv, f.chunks, sub, mask, top_k >> 31) : quad_dot(plane, qv, f.chunks, sub, mask);
+                nd = f.nodes[above_from_dot(d, f.cst[nd.x]) ? nd.z : nd.y];
+            }
+            if (f.leaf_plan[nd.w] > 0) {
+                if (nvis < cap && sub == 0) wvisits[(size_t)w * vpw + 1 + nvis] = make_uint2((u32)nd.w, top_k);
+                ++nvis;
+            }
+        }
     }
     if (sub == 0) {
         if (nvis > cap && !ovf) ovf = 1;
@@ -144,21 +243,51 @@ __global__ void __launch_bounds__(128, 1) plan_walk_tail_kernel(ForestView f, co
     for (u32 i = blockIdx.x * 32u + (threadIdx.x >> 2); i < n; i += gridDim.x * 32u)
         plan_walk_one<true>(f, queries, tail_list[i], (int)(threadIdx.x & 3), mask, top_k, vpw, wvisits, wcounts, overflow, nullptr, nullptr);
 }
+// The same two kernels for a multi-probe batch (probes >= 1).
+__global__ void __launch_bounds__(128) plan_walk_probe_kernel(ForestView f, const float* __restrict__ queries, u32 nq, u32 top_k,
+                                                              u32 probes, u32 vpw, uint2* __restrict__ wvisits,
+                                                              u32* __restrict__ wcounts, u32* __restrict__ overflow,
+                                                              u32* __restrict__ tail_list, u32* __restrict__ tail_count) {
+    const u32 w = blockIdx.x * 32u + (threadIdx.x >> 2);
+    const u32 nwalkers = nq * (u32)f.num_trees;
+    if (w >= nwalkers) return;
+    plan_walk_one<false, true>(f, queries, w, (int)(threadIdx.x & 3), quad_mask(), top_k, vpw, wvisits, wcounts, overflow, tail_list,
+                               tail_count, probes);
+}
+__global__ void __launch_bounds__(128, 1) plan_walk_probe_tail_kernel(ForestView f, const float* __restrict__ queries, u32 top_k,
+                                                                      u32 probes, u32 vpw, uint2* __restrict__ wvisits,
+                                                                      u32* __restrict__ wcounts, u32* __restrict__ overflow,
+                                                                      const u32* __restrict__ tail_list,
+                                                                      const u32* __restrict__ tail_count) {
+    const u32 n = *tail_count;
+    const unsigned mask = quad_mask();
+    for (u32 i = blockIdx.x * 32u + (threadIdx.x >> 2); i < n; i += gridDim.x * 32u)
+        plan_walk_one<true, true>(f, queries, tail_list[i], (int)(threadIdx.x & 3), mask, top_k, vpw, wvisits, wcounts, overflow, nullptr,
+                                  nullptr, probes);
+}
 
 // tail_list: [walkers + 1] u32 scratch, element 0 is the counter; pass nullptr to keep every walker in the main kernel (what a
-// forest whose leaves cannot hold top_k rows wants: there every walker cascades).
-void launch_plan(const ForestView& f, const float* d_queries, u32 nq, u32 top_k, u32 vpw, uint2* d_wvisits,
+// forest whose leaves cannot hold top_k rows wants: there every walker cascades).  probes > 0: the multi-probe walk.
+void launch_plan(const ForestView& f, const float* d_queries, u32 nq, u32 top_k, u32 probes, u32 vpw, uint2* d_wvisits,
                  u32* d_wcounts, u32* d_overflow, u32* d_tail_list, cudaStream_t s) {
     u32 nwalkers = nq * (u32)f.num_trees;
     if (!nwalkers) return;
     if (d_tail_list) cudaMemsetAsync(d_tail_list, 0, 4, s);
-    plan_walk_kernel<<<(nwalkers + 31) / 32, 128, 0, s>>>(f, d_queries, nq, top_k, vpw, d_wvisits, d_wcounts, d_overflow,
-                                                          d_tail_list ? d_tail_list + 1 : nullptr, d_tail_list);
+    if (probes)
+        plan_walk_probe_kernel<<<(nwalkers + 31) / 32, 128, 0, s>>>(f, d_queries, nq, top_k, probes, vpw, d_wvisits, d_wcounts, d_overflow,
+                                                                    d_tail_list ? d_tail_list + 1 : nullptr, d_tail_list);
+    else
+        plan_walk_kernel<<<(nwalkers + 31) / 32, 128, 0, s>>>(f, d_queries, nq, top_k, vpw, d_wvisits, d_wcounts, d_overflow,
+                                                              d_tail_list ? d_tail_list + 1 : nullptr, d_tail_list);
     if (d_tail_list) {
         int dev = 0, sms = 0;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        plan_walk_tail_kernel<<<sms * 2, 128, 0, s>>>(f, d_queries, top_k, vpw, d_wvisits, d_wcounts, d_overflow, d_tail_list + 1, d_tail_list);
+        if (probes)
+            plan_walk_probe_tail_kernel<<<sms * 2, 128, 0, s>>>(f, d_queries, top_k, probes, vpw, d_wvisits, d_wcounts, d_overflow,
+                                                                d_tail_list + 1, d_tail_list);
+        else
+            plan_walk_tail_kernel<<<sms * 2, 128, 0, s>>>(f, d_queries, top_k, vpw, d_wvisits, d_wcounts, d_overflow, d_tail_list + 1, d_tail_list);
     }
 }
 

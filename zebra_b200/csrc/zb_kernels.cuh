@@ -53,7 +53,7 @@ struct RecvSeg {      // rows of one (source rank, owned leaf) pair in the recei
 };
 
 // ---- plan (tree_result control flow, lsh.rs:290-348) ----
-void launch_plan(const ForestView& f, const float* d_queries, u32 nq, u32 top_k, u32 vpw, uint2* d_wvisits,
+void launch_plan(const ForestView& f, const float* d_queries, u32 nq, u32 top_k, u32 probes, u32 vpw, uint2* d_wvisits,
                  u32* d_wcounts, u32* d_overflow, u32* d_tail_list, cudaStream_t s);
 // sharded plan exchange (compacted visit records, header first): pack -> ncclAllGather -> flags -> scan -> scatter -> offsets
 void launch_pack_visits(u32 nwalkers, u32 vpw, const uint2* d_wvisits, const u32* d_wcounts, const u32* d_woff, u32 walker_base,

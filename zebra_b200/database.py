@@ -103,11 +103,12 @@ class Database:
             return {}
         return self.query_vectors(self.model.embed_documents(documents), number_of_results)
 
-    def query_vectors(self, vectors, number_of_results: int) -> Dict[int, Dict[_uuid.UUID, bytes]]:  # core.rs:290-313
+    def query_vectors(self, vectors, number_of_results: int, probes: int = 0) -> Dict[int, Dict[_uuid.UUID, bytes]]:  # core.rs:290-313
+        """probes > 0: multi-probe search (LSHIndex.search_batch); 0 is the reference's query."""
         if self.index.no_vectors():
             return {}
         vectors = np.ascontiguousarray(vectors, dtype=np.float32).reshape(-1, self.dim)
-        ids, _, _, counts = self.index.search_batch(vectors, number_of_results)  # ONE batched device call
+        ids, _, _, counts = self.index.search_batch(vectors, number_of_results, probes=probes)  # ONE batched device call
         out: Dict[int, Dict[_uuid.UUID, bytes]] = {}
         for q in range(vectors.shape[0]):
             out[q] = {i: self._documents.get(i, b"") for i in _bytes_to_ids(ids[q, : int(counts[q])])}

@@ -165,14 +165,16 @@ class LSHIndex:
         return self.no_vectors() or self.no_trees()
 
     # ---------------------------------------------------------------- lsh.rs:544-565
-    def search(self, query, top_k: int, metric: Optional[_DeviceMetric] = None) -> List[Tuple[_uuid.UUID, int]]:
+    # probes (every search form): 0 = the reference's search; P > 0 also visits, in every tree, the leaves across the P
+    # main-path planes closest to the query (multi-probe, DESIGN 3.9; at most ZB_MAX_PROBES = 32)
+    def search(self, query, top_k: int, metric: Optional[_DeviceMetric] = None, probes: int = 0) -> List[Tuple[_uuid.UUID, int]]:
         if metric is not None and metric != self.metric:
             raise ValueError("this device index was created for " + type(self.metric).__name__)
-        ids, _, bits, counts = self.search_batch(np.asarray(query, np.float32)[None, :], top_k)
+        ids, _, bits, counts = self.search_batch(np.asarray(query, np.float32)[None, :], top_k, probes=probes)
         c = int(counts[0])
         return list(zip(_bytes_to_ids(ids[0, :c]), (int(b) for b in bits[0, :c])))
 
-    def search_batch(self, queries, top_k: int, want_ids: bool = True):
+    def search_batch(self, queries, top_k: int, want_ids: bool = True, probes: int = 0):
         """One call for the whole batch (replaces the par_iter of core.rs:299).  Returns
         (ids [nq,k,16] uint8 or None, ordinals [nq,k] uint64, distance bits [nq,k] uint64, counts [nq] uint32)."""
         q = np.ascontiguousarray(queries, dtype=np.float32).reshape(-1, self.dim)
@@ -181,18 +183,25 @@ class LSHIndex:
         ords = np.empty((nq, top_k), dtype=np.uint64)
         bits = np.empty((nq, top_k), dtype=np.uint64)
         counts = np.zeros(nq, dtype=np.uint32)
-        _ffi.check(_ffi.lib().zb_index_search_batch(self._h, nq, q.ctypes.data, top_k,
-                                                    ids.ctypes.data if want_ids else None, ords.ctypes.data,
-                                                    bits.ctypes.data, counts.ctypes.data))
+        self.search_batch_ptr(nq, q.ctypes.data, top_k, ords.ctypes.data, bits.ctypes.data, counts.ctypes.data,
+                              ids.ctypes.data if want_ids else None, probes=probes)
         return ids, ords, bits, counts
 
     def search_batch_ptr(self, nq: int, q_ptr: int, top_k: int, ord_ptr: int, bits_ptr: int, counts_ptr: int,
-                         ids_ptr: Optional[int] = None) -> None:
+                         ids_ptr: Optional[int] = None, probes: int = 0) -> None:
         """Host-pointer form (e.g. pinned buffers owned by the caller)."""
-        _ffi.check(_ffi.lib().zb_index_search_batch(self._h, nq, q_ptr, top_k, ids_ptr, ord_ptr, bits_ptr, counts_ptr))
+        if probes:
+            _ffi.check(_ffi.lib().zb_index_search_probe(self._h, nq, q_ptr, top_k, probes, ids_ptr, ord_ptr, bits_ptr, counts_ptr))
+        else:
+            _ffi.check(_ffi.lib().zb_index_search_batch(self._h, nq, q_ptr, top_k, ids_ptr, ord_ptr, bits_ptr, counts_ptr))
 
-    def search_batch_device(self, nq: int, d_q_ptr: int, top_k: int, d_ord_ptr: int, d_bits_ptr: int, d_counts_ptr: int):
-        _ffi.check(_ffi.lib().zb_index_search_batch_device(self._h, nq, d_q_ptr, top_k, d_ord_ptr, d_bits_ptr, d_counts_ptr))
+    def search_batch_device(self, nq: int, d_q_ptr: int, top_k: int, d_ord_ptr: int, d_bits_ptr: int, d_counts_ptr: int,
+                            probes: int = 0):
+        if probes:
+            _ffi.check(_ffi.lib().zb_index_search_probe_device(self._h, nq, d_q_ptr, top_k, probes, d_ord_ptr, d_bits_ptr,
+                                                               d_counts_ptr))
+        else:
+            _ffi.check(_ffi.lib().zb_index_search_batch_device(self._h, nq, d_q_ptr, top_k, d_ord_ptr, d_bits_ptr, d_counts_ptr))
 
     # ---------------------------------------------------------------- exact (brute-force) search, zb_index_search_exact
     def search_exact(self, query, top_k: int) -> List[Tuple[_uuid.UUID, int]]:
@@ -225,7 +234,7 @@ class LSHIndex:
         lo = min(nq_total, shard_rank * nqp)
         return lo, min(nq_total, lo + nqp)
 
-    def search_slice(self, nq_total: int, slice_queries, top_k: int, want_ids: bool = True):
+    def search_slice(self, nq_total: int, slice_queries, top_k: int, want_ids: bool = True, probes: int = 0):
         """Collective.  `slice_queries` = this rank's slice of the batch; returns that slice's (ids, ordinals, bits, counts)."""
         q = np.ascontiguousarray(slice_queries, dtype=np.float32).reshape(-1, self.dim)
         n = q.shape[0]
@@ -233,21 +242,30 @@ class LSHIndex:
         ords = np.empty((n, top_k), dtype=np.uint64)
         bits = np.empty((n, top_k), dtype=np.uint64)
         counts = np.zeros(n, dtype=np.uint32)
-        _ffi.check(_ffi.lib().zb_index_search_slice(self._h, nq_total, q.ctypes.data if n else None, top_k,
-                                                    ids.ctypes.data if want_ids and n else None, ords.ctypes.data if n else None,
-                                                    bits.ctypes.data if n else None, counts.ctypes.data if n else None))
+        self.search_slice_ptr(nq_total, q.ctypes.data if n else None, top_k, ords.ctypes.data if n else None,
+                              bits.ctypes.data if n else None, counts.ctypes.data if n else None,
+                              ids.ctypes.data if want_ids and n else None, probes=probes)
         return ids, ords, bits, counts
 
     def search_slice_ptr(self, nq_total: int, q_ptr: int, top_k: int, ord_ptr: int, bits_ptr: int, counts_ptr: int,
-                         ids_ptr: Optional[int] = None) -> None:
-        _ffi.check(_ffi.lib().zb_index_search_slice(self._h, nq_total, q_ptr, top_k, ids_ptr, ord_ptr, bits_ptr, counts_ptr))
+                         ids_ptr: Optional[int] = None, probes: int = 0) -> None:
+        if probes:
+            _ffi.check(_ffi.lib().zb_index_search_slice_probe(self._h, nq_total, q_ptr, top_k, probes, ids_ptr, ord_ptr, bits_ptr,
+                                                              counts_ptr))
+        else:
+            _ffi.check(_ffi.lib().zb_index_search_slice(self._h, nq_total, q_ptr, top_k, ids_ptr, ord_ptr, bits_ptr, counts_ptr))
 
     def search_prefetch_ptr(self, n: int, q_ptr: int):
         """Announce the next batch (zb_index_search_prefetch): its upload overlaps the search call in between."""
         _ffi.check(_ffi.lib().zb_index_search_prefetch(self._h, n, q_ptr))
 
-    def search_slice_device(self, nq_total: int, d_q_ptr: int, top_k: int, d_ord_ptr: int, d_bits_ptr: int, d_counts_ptr: int):
-        _ffi.check(_ffi.lib().zb_index_search_slice_device(self._h, nq_total, d_q_ptr, top_k, d_ord_ptr, d_bits_ptr, d_counts_ptr))
+    def search_slice_device(self, nq_total: int, d_q_ptr: int, top_k: int, d_ord_ptr: int, d_bits_ptr: int, d_counts_ptr: int,
+                            probes: int = 0):
+        if probes:
+            _ffi.check(_ffi.lib().zb_index_search_slice_probe_device(self._h, nq_total, d_q_ptr, top_k, probes, d_ord_ptr,
+                                                                     d_bits_ptr, d_counts_ptr))
+        else:
+            _ffi.check(_ffi.lib().zb_index_search_slice_device(self._h, nq_total, d_q_ptr, top_k, d_ord_ptr, d_bits_ptr, d_counts_ptr))
 
     # ---------------------------------------------------------------- bucket keys
     def hash(self, rows):
