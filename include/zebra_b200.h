@@ -211,6 +211,55 @@ int zb_index_search_slice_probe_device(zb_index* index, uint64_t nq_total, const
                                        uint32_t probes, uint64_t* d_out_ordinals, uint64_t* d_out_dist_bits,
                                        uint32_t* d_out_counts);
 
+/* Restricted search (DESIGN.md 3.10): run a search over a caller-given set of rows, as if every other row had been removed
+ * -- one tenant's documents, the rows a permission check allows, everything but what a user has already seen -- without
+ * changing the index for any other caller.
+ *   - A rowset is a fixed set of ordinals, fixed when it is made from a list of ordinals or ids: the listed rows, or with
+ *     ZB_ROWSET_EXCLUDE every ordinal < total_rows at creation except the listed ones.  Duplicate list entries are allowed;
+ *     rows added later are never in a rowset.  *out_count (NULL-able) receives the number of ordinals in the set.
+ *   - An ordinal >= total_rows returns ZB_ERR_INVALID (the _device form checks on the device); from ids, an unknown id sets
+ *     out_found[i] = 0 (NULL-able) and is ignored.  Any flag bit other than ZB_ROWSET_EXCLUDE returns ZB_ERR_INVALID.
+ *   - Restricted search with rowset R is the plain search on the index's current state with every live row outside R treated
+ *     as removed (D1): leaves count only the live rows of R (cascade Q1, per-visit n' of Q2, the probe rule of 3.9 over the
+ *     same counts), only those rows become candidates, in zb_index_search_batch's order (literal cosine Q4).  This holds for
+ *     every metric and scan path, probes 0..ZB_MAX_PROBES, the whole-batch and sliced forms, and the exact search (which
+ *     returns the exact top_k over the live rows of R).
+ *   - Coverage is taken at call time: rows removed after the rowset was made are excluded; inserts (and the leaf splits they
+ *     cause) and zb_index_deduplicate are taken into account.  zb_index_clear, zb_index_load_forest, zb_index_load_flat and
+ *     zb_index_import_store reuse ordinals: afterwards a rowset made earlier returns ZB_ERR_STATE.  A rowset of another index
+ *     returns ZB_ERR_INVALID; rowset = NULL is the unrestricted call.
+ *   - A rowset belongs to its index and holds device memory (a bit per ordinal, and what the first restricted call derives
+ *     from it; counted in zb_stats.device_bytes): destroy it before the index.
+ *   - Sharded index: every rank makes the rowset from the same list, as with zb_index_add; restricted searches are collective
+ *     like the plain ones.
+ *   - zb_stats describes a restricted LSH batch like any other; the restricted exact search leaves zb_stats alone.  The first
+ *     restricted batch after the index changed (or the first one of a rowset) derives the rowset's masks and leaf counts inside
+ *     its timed window: that work is part of its last_ms_plan and last_ms_total.
+ * Layout, 0xFF tail fill, NULL-able outputs and the limits on top_k / probes are those of the plain calls. */
+typedef struct zb_rowset zb_rowset;
+#define ZB_ROWSET_EXCLUDE 1u
+int zb_index_rowset_from_ordinals(zb_index* index, uint64_t n, const uint64_t* ordinals, uint32_t flags, uint64_t* out_count,
+                                  zb_rowset** out_rowset);
+int zb_index_rowset_from_ordinals_device(zb_index* index, uint64_t n, const uint64_t* d_ordinals, uint32_t flags,
+                                         uint64_t* out_count, zb_rowset** out_rowset);
+int zb_index_rowset_from_ids(zb_index* index, uint64_t n, const uint8_t* ids16, uint32_t flags, uint8_t* out_found,
+                             uint64_t* out_count, zb_rowset** out_rowset);
+int zb_rowset_destroy(zb_rowset* rowset);
+int zb_index_search_rowset(zb_index* index, uint64_t nq, const float* queries, uint64_t top_k, uint32_t probes, zb_rowset* rowset,
+                           uint8_t* out_ids16, uint64_t* out_ordinals, uint64_t* out_dist_bits, uint32_t* out_counts);
+int zb_index_search_rowset_device(zb_index* index, uint64_t nq, const float* d_queries, uint64_t top_k, uint32_t probes,
+                                  zb_rowset* rowset, uint64_t* d_out_ordinals, uint64_t* d_out_dist_bits, uint32_t* d_out_counts);
+int zb_index_search_slice_rowset(zb_index* index, uint64_t nq_total, const float* slice_queries, uint64_t top_k, uint32_t probes,
+                                 zb_rowset* rowset, uint8_t* out_ids16, uint64_t* out_ordinals, uint64_t* out_dist_bits,
+                                 uint32_t* out_counts);
+int zb_index_search_slice_rowset_device(zb_index* index, uint64_t nq_total, const float* d_slice_queries, uint64_t top_k,
+                                        uint32_t probes, zb_rowset* rowset, uint64_t* d_out_ordinals, uint64_t* d_out_dist_bits,
+                                        uint32_t* d_out_counts);
+int zb_index_search_exact_rowset(zb_index* index, uint64_t nq, const float* queries, uint64_t top_k, zb_rowset* rowset,
+                                 uint8_t* out_ids16, uint64_t* out_ordinals, uint64_t* out_dist_bits, uint32_t* out_counts);
+int zb_index_search_exact_rowset_device(zb_index* index, uint64_t nq, const float* d_queries, uint64_t top_k, zb_rowset* rowset,
+                                        uint64_t* d_out_ordinals, uint64_t* d_out_dist_bits, uint32_t* d_out_counts);
+
 /* Bucket keys: the root-to-leaf sign path of Hyperplane::point_is_above decisions (lsh.rs:39-43 along
  * :350-366), MSB = root, 1 = above/right, for every (row, tree): out_keys/out_depths/out_leaves are
  * [n][num_trees] (a path longer than 64 keeps its last 64 bits; out_leaves is the leaf number of

@@ -288,22 +288,78 @@ class LSHIndex {
     /// bits, id), at most top_k entries.
     std::vector<std::vector<std::pair<Uuid, DistanceUnit>>> search_batch(const std::vector<Embedding<N>>& queries, size_t top_k,
                                                                          uint32_t probes = 0) const {
-        const size_t nq = queries.size();
-        std::vector<uint8_t> ids(nq * top_k * 16 + 1);
-        std::vector<uint64_t> bits(nq * top_k + 1);
-        std::vector<uint32_t> counts(nq + 1, 0);
-        if (probes)
-            check(zb_index_search_probe(raw(), nq, nq ? queries[0].data() : nullptr, top_k, probes, ids.data(), nullptr, bits.data(),
-                                        counts.data()));
-        else
-            check(zb_index_search_batch(raw(), nq, nq ? queries[0].data() : nullptr, top_k, ids.data(), nullptr, bits.data(), counts.data()));
-        std::vector<std::vector<std::pair<Uuid, DistanceUnit>>> out(nq);
-        for (size_t q = 0; q < nq; ++q)
-            for (uint32_t i = 0; i < counts[q]; ++i) {
-                const size_t o = q * top_k + i;
-                out[q].emplace_back(Uuid::from_slice(ids.data() + 16 * o), bits[o]);
+        return run_search(queries, top_k, [&](uint64_t nq, const float* q, uint8_t* ids, uint64_t* bits, uint32_t* counts) {
+            return probes ? zb_index_search_probe(raw(), nq, q, top_k, probes, ids, nullptr, bits, counts)
+                          : zb_index_search_batch(raw(), nq, q, top_k, ids, nullptr, bits, counts);
+        });
+    }
+
+    /// A fixed set of rows of this index for restricted search (zb_index_rowset_*, DESIGN 3.10): a search `within` it returns
+    /// what the plain search returns with every live row outside the set removed.  Owns the zb_rowset; keeps the index alive.
+    class RowSet {
+        friend class LSHIndex;
+        std::shared_ptr<Handle> ix_;
+        zb_rowset* p_ = nullptr;
+        uint64_t count_ = 0;
+
+      public:
+        RowSet() = default;
+        RowSet(RowSet&& o) noexcept : ix_(std::move(o.ix_)), p_(o.p_), count_(o.count_) { o.p_ = nullptr; }
+        RowSet& operator=(RowSet&& o) noexcept {
+            if (this != &o) {
+                reset();
+                ix_ = std::move(o.ix_);
+                p_ = o.p_;
+                count_ = o.count_;
+                o.p_ = nullptr;
             }
-        return out;
+            return *this;
+        }
+        RowSet(const RowSet&) = delete;
+        RowSet& operator=(const RowSet&) = delete;
+        ~RowSet() { reset(); }
+        void reset() {
+            if (p_) zb_rowset_destroy(p_);
+            p_ = nullptr;
+        }
+        zb_rowset* raw() const { return p_; }
+        uint64_t count() const { return count_; }  /// ordinals in the set
+    };
+    /// The rows with these ids (exclude: every row present now except them); unknown ids are ignored (found[i] = 0).
+    RowSet rowset(const std::vector<Uuid>& ids, bool exclude = false, std::vector<uint8_t>* found = nullptr) const {
+        std::vector<uint8_t> raw_ids = pack(ids), f(ids.size() + 1, 0);
+        RowSet rs;
+        rs.ix_ = h_;
+        check(zb_index_rowset_from_ids(raw(), ids.size(), raw_ids.data(), exclude ? ZB_ROWSET_EXCLUDE : 0u, f.data(), &rs.count_, &rs.p_));
+        if (found) found->assign(f.begin(), f.begin() + ids.size());
+        return rs;
+    }
+    /// The same from ordinals; an ordinal >= total_rows throws (ZB_ERR_INVALID).
+    RowSet rowset_ordinals(const std::vector<uint64_t>& ordinals, bool exclude = false) const {
+        RowSet rs;
+        rs.ix_ = h_;
+        check(zb_index_rowset_from_ordinals(raw(), ordinals.size(), ordinals.data(), exclude ? ZB_ROWSET_EXCLUDE : 0u, &rs.count_, &rs.p_));
+        return rs;
+    }
+    /// search_batch restricted to `within`.
+    std::vector<std::vector<std::pair<Uuid, DistanceUnit>>> search_batch(const std::vector<Embedding<N>>& queries, size_t top_k,
+                                                                         const RowSet& within, uint32_t probes = 0) const {
+        return run_search(queries, top_k, [&](uint64_t nq, const float* q, uint8_t* ids, uint64_t* bits, uint32_t* counts) {
+            return zb_index_search_rowset(raw(), nq, q, top_k, probes, live(within), ids, nullptr, bits, counts);
+        });
+    }
+    /// Exact search (zb_index_search_exact): the true top_k over every live row, in search_batch's order.
+    std::vector<std::vector<std::pair<Uuid, DistanceUnit>>> search_exact(const std::vector<Embedding<N>>& queries, size_t top_k) const {
+        return run_search(queries, top_k, [&](uint64_t nq, const float* q, uint8_t* ids, uint64_t* bits, uint32_t* counts) {
+            return zb_index_search_exact(raw(), nq, q, top_k, ids, nullptr, bits, counts);
+        });
+    }
+    /// The exact top_k over the live rows of `within`.
+    std::vector<std::vector<std::pair<Uuid, DistanceUnit>>> search_exact(const std::vector<Embedding<N>>& queries, size_t top_k,
+                                                                         const RowSet& within) const {
+        return run_search(queries, top_k, [&](uint64_t nq, const float* q, uint8_t* ids, uint64_t* bits, uint32_t* counts) {
+            return zb_index_search_exact_rowset(raw(), nq, q, top_k, live(within), ids, nullptr, bits, counts);
+        });
     }
 
     /// Bucket keys (root-to-leaf sign path of lsh.rs:350-366, MSB = root): keys[i * num_trees + t], depths likewise.
@@ -383,6 +439,11 @@ class LSHIndex {
     }
 
   private:
+    // the C ABI takes a NULL rowset as the unrestricted search: an empty (default, moved-from or reset) RowSet is refused
+    static zb_rowset* live(const RowSet& within) {
+        if (!within.raw()) throw Error(ZB_ERR_INVALID, "search within an empty RowSet");
+        return within.raw();
+    }
     static std::vector<uint8_t> pack(const std::vector<Uuid>& ids) {
         std::vector<uint8_t> raw_ids(ids.size() * 16 + 1);
         for (size_t i = 0; i < ids.size(); ++i) std::memcpy(raw_ids.data() + 16 * i, ids[i].bytes.data(), 16);
@@ -396,6 +457,23 @@ class LSHIndex {
         std::vector<Uuid> res;
         for (size_t i = 0; i < n; ++i) res.push_back(Uuid::from_slice(out.data() + 16 * i));
         return res;
+    }
+    // host buffers for one batched search call `call(nq, queries, ids, bits, counts)`, and its per-query (id, bits) lists
+    template <class Call>
+    std::vector<std::vector<std::pair<Uuid, DistanceUnit>>> run_search(const std::vector<Embedding<N>>& queries, size_t top_k,
+                                                                       Call call) const {
+        const size_t nq = queries.size();
+        std::vector<uint8_t> ids(nq * top_k * 16 + 1);
+        std::vector<uint64_t> bits(nq * top_k + 1);
+        std::vector<uint32_t> counts(nq + 1, 0);
+        check(call(nq, nq ? queries[0].data() : nullptr, ids.data(), bits.data(), counts.data()));
+        std::vector<std::vector<std::pair<Uuid, DistanceUnit>>> out(nq);
+        for (size_t q = 0; q < nq; ++q)
+            for (uint32_t i = 0; i < counts[q]; ++i) {
+                const size_t o = q * top_k + i;
+                out[q].emplace_back(Uuid::from_slice(ids.data() + 16 * o), bits[o]);
+            }
+        return out;
     }
 };
 

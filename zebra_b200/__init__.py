@@ -10,10 +10,10 @@ from .database import Database, DatabaseEmbeddingModel
 from .distance import (BrayCurtisDistance, CanberraDistance, ChebyshevDistance, CosineDistance, HammingDistance,
                        L2Distance, L2SquaredDistance, L3Distance, L4Distance, ManhattanDistance, MinkowskiDistance,
                        PNormDistance, bits_to_f64, f64_to_bits, point_is_above)
-from .index import Forest, LSHIndex, LSHIndexOptions, comm_unique_id, recall_at_k, synth_fill_device
+from .index import Forest, LSHIndex, LSHIndexOptions, RowSet, comm_unique_id, recall_at_k, synth_fill_device
 
 __all__ = [
-    "Database", "DatabaseEmbeddingModel", "LSHIndex", "LSHIndexOptions", "Forest", "CosineDistance", "L2Distance",
+    "Database", "DatabaseEmbeddingModel", "LSHIndex", "LSHIndexOptions", "RowSet", "Forest", "CosineDistance", "L2Distance",
     "L2SquaredDistance", "ChebyshevDistance", "CanberraDistance", "BrayCurtisDistance", "ManhattanDistance", "L3Distance",
     "L4Distance", "HammingDistance", "MinkowskiDistance", "PNormDistance", "ZebraError", "bits_to_f64", "f64_to_bits", "point_is_above", "comm_unique_id",
     "synth_fill_device", "recall_at_k",

@@ -118,6 +118,16 @@ SYMBOLS = {
     "zb_index_search_probe_device": (C.c_int, [_vp, _u64, _vp, _u64, C.c_uint32, _vp, _vp, _vp]),
     "zb_index_search_slice_probe": (C.c_int, [_vp, _u64, _vp, _u64, C.c_uint32, _vp, _vp, _vp, _vp]),
     "zb_index_search_slice_probe_device": (C.c_int, [_vp, _u64, _vp, _u64, C.c_uint32, _vp, _vp, _vp]),
+    "zb_index_rowset_from_ordinals": (C.c_int, [_vp, _u64, _vp, _u32, C.POINTER(_u64), C.POINTER(_vp)]),
+    "zb_index_rowset_from_ordinals_device": (C.c_int, [_vp, _u64, _vp, _u32, C.POINTER(_u64), C.POINTER(_vp)]),
+    "zb_index_rowset_from_ids": (C.c_int, [_vp, _u64, _vp, _u32, _vp, C.POINTER(_u64), C.POINTER(_vp)]),
+    "zb_rowset_destroy": (C.c_int, [_vp]),
+    "zb_index_search_rowset": (C.c_int, [_vp, _u64, _vp, _u64, _u32, _vp, _vp, _vp, _vp, _vp]),
+    "zb_index_search_rowset_device": (C.c_int, [_vp, _u64, _vp, _u64, _u32, _vp, _vp, _vp, _vp]),
+    "zb_index_search_slice_rowset": (C.c_int, [_vp, _u64, _vp, _u64, _u32, _vp, _vp, _vp, _vp, _vp]),
+    "zb_index_search_slice_rowset_device": (C.c_int, [_vp, _u64, _vp, _u64, _u32, _vp, _vp, _vp, _vp]),
+    "zb_index_search_exact_rowset": (C.c_int, [_vp, _u64, _vp, _u64, _vp, _vp, _vp, _vp, _vp]),
+    "zb_index_search_exact_rowset_device": (C.c_int, [_vp, _u64, _vp, _u64, _vp, _vp, _vp, _vp]),
     "zb_index_hash": (C.c_int, [_vp, _u64, _vp, _vp, _vp, _vp]),
     "zb_index_hash_device": (C.c_int, [_vp, _u64, _vp, _vp, _vp, _vp]),
     "zb_index_forest_sizes": (C.c_int, [_vp, _vp]),

@@ -7,6 +7,7 @@
 // every dot product, distance, sign test, partition and top-k runs in a CUDA kernel.
 #include <algorithm>
 #include <chrono>
+#include <memory>
 #include <mutex>
 #include <unordered_map>
 
@@ -196,6 +197,11 @@ struct zb_index {
     DBuf<double> ex_rinv;
     DBuf<float> ex_n2;
     DBuf<u64> ex_loc, ex_gath, ex_nmax;
+    // restricted search (zb_rowset): mut_gen changes with every call that changes tombstones, rows, the forest or the
+    // bucket-major store (a rowset's masks and leaf counts derived under another value are stale); content_epoch changes
+    // when ordinals are reused (clear, and the loads that start with one), which invalidates every rowset made before.
+    // On a sharded index both move in the same calls on every rank: those calls are collective.
+    u64 mut_gen = 0, content_epoch = 0;
 
     // ---- knobs / stats ----
     int64_t p_tile_min_rows = 64, p_tile_queries = 0, p_use_tile_scan = 1, p_hash_variant = 0, p_classify_variant = 0, p_seq_tile = 1, p_seq_prefetch = 0, p_flat_project = 1, p_quad_tile = 1, p_select_variant = 1, p_scan_gen = 3, p_bm_stage_mb = 2048, p_single_exchange = 1, p_p2p_queries = 1, p_l2_filter = 1, p_plan_tail = 1, p_exact_budget_mb = 256;
@@ -388,6 +394,7 @@ struct zb_index {
         sync();
         export_table_valid = false;
         bm_valid = false;
+        ++mut_gen;
     }
     // (Re)build the bucket-major store after the forest or the row set changed.  Only forests whose leaves can reach
     // the tile kernel's minimum size get one; an allocation failure degrades to the generic gather path.
@@ -432,6 +439,7 @@ struct zb_index {
         sync();
         bm_positions = members_used;
         bm_valid = true;
+        ++mut_gen;
         return true;
     }
     // Bucket-sharded store (north_star (c), SURVEY 8e): every leaf is moved, whole, to rank leaf % G -- each rank packs
@@ -612,6 +620,7 @@ struct zb_index {
         sync();
         bm_positions = P;
         bm_valid = true;
+        ++mut_gen;
         return true;
     }
     // Collective (every rank calls it with the same `need`): (re)allocates the batch buffer, exchanges the IPC handles through
@@ -713,6 +722,7 @@ struct zb_index {
         d_leaf_plan.ensure(nl ? nl : 1);
         if (nl) count_live_kernel<<<(nl + 127) / 128, 128, 0, stream>>>(d_members.p, d_leaf_off.p, d_leaf_len.p, tomb.p, nl, d_leaf_live.p);
         refresh_plan_counts();
+        ++mut_gen;
     }
     void refresh_plan_counts() {
         u32 nl = (u32)h_leaf_off.size();
@@ -988,18 +998,115 @@ struct zb_index {
     }
 };
 
+// A fixed set of global ordinals (zb_index_rowset_*) and what a restricted search derives from it.  Restricted search with
+// rowset R is the plain search with every live row outside R taken as removed (D1), so it substitutes three arrays of the
+// plain search and changes nothing else: the slot tombstones, the bucket-major tombstones and the per-leaf live counts.
+struct zb_rowset {
+    zb_index* ix = nullptr;
+    u64 epoch = 0;     // ix->content_epoch at creation
+    u64 nbits = 0;     // total_rows at creation: later rows are never in the set
+    u64 count = 0;     // ordinals in the set
+    DBuf<u32> bits;    // bit o = ordinal o is in the set (the whole bitmap on every rank of a sharded index)
+    // derived, valid while gen == ix->mut_gen: slot mask = tomb | ~in(ordinal of slot), the same over bucket-major positions
+    // (when the index has a store), the leaf counts of the rows either leaves in (sharded: summed over the ranks)
+    u64 gen = ~0ull;
+    DBuf<u32> slot_mask, bm_mask, leaf_live, leaf_plan;
+    DBuf<u64> d_live;
+    u64 n_live = 0;    // slots of this rank the slot mask leaves in
+    // exact search, compacted side of the half rule: the rows of the set live when it was gathered, ordinals ascending, their
+    // side arrays, and a mask over them refreshed from the slot mask whenever the index changed (c_gen != gen)
+    bool compact = false;
+    u64 c_n = 0, c_gen = ~0ull;
+    DBuf<float> c_rows, c_n2;
+    DBuf<u64> c_ord;
+    DBuf<u32> c_slot, c_mask;
+    DBuf<double> c_rinv;
+};
+
 // =====================================================================================================
 // search
 // =====================================================================================================
 namespace zb {
+
+static void rowset_check(zb_index* ix, const zb_rowset* rs) {
+    ZB_REQUIRE(rs->ix == ix, ZB_ERR_INVALID, "rowset of another index");
+    ZB_REQUIRE(rs->epoch == ix->content_epoch, ZB_ERR_STATE, "rowset made before the index was cleared or reloaded");
+}
+
+// (Re)derives the rowset's masks and leaf counts if the index changed since the last restricted call.  Call after
+// ensure_bucket_major (a search may rebuild the store).  Sharded: collective (the leaf counts are summed over the ranks);
+// every rank sees the same changes, so every rank recomputes in the same call.
+static void rowset_derive(zb_index* ix, zb_rowset* rs) {
+    if (rs->gen == ix->mut_gen) return;
+    cudaStream_t s = ix->stream;
+    const u64 sw = ix->n_slots / 32 + 8;   // + 8: the scan kernels read tombstone words past a block's last position
+    rs->slot_mask.ensure(sw);
+    rs->d_live.ensure(1);
+    ZB_CUDA(cudaMemsetAsync(rs->d_live.p, 0, 8, s));
+    launch_rowset_mask(ix->ord.p, ix->n_slots, ix->tomb.p, rs->bits.p, rs->nbits, 0, sw, rs->slot_mask.p, rs->d_live.p, s);
+    const u32 nl = (u32)ix->h_leaf_off.size();
+    rs->leaf_live.ensure(nl ? nl : 1);
+    if (nl)
+        count_live_kernel<<<(nl + 127) / 128, 128, 0, s>>>(ix->d_members.p, ix->d_leaf_off.p, ix->d_leaf_len.p, rs->slot_mask.p, nl,
+                                                           rs->leaf_live.p);
+    if (ix->G > 1 && nl) {
+        rs->leaf_plan.ensure(nl);
+        ZB_CUDA(cudaMemcpyAsync(rs->leaf_plan.p, rs->leaf_live.p, (size_t)nl * 4, cudaMemcpyDeviceToDevice, s));
+        ix->nccl.allreduce(rs->leaf_plan.p, nl, Nccl::U32, Nccl::SUM, s);
+    }
+    if (ix->bm_valid) {   // the ordinal at a position: the member slot unsharded (slot == ordinal), bm_ord sharded
+        const u64 bw = ix->bm_positions / 32 + 8;
+        rs->bm_mask.ensure(bw);
+        if (ix->G > 1)
+            launch_rowset_mask(ix->bm_ord.p, ix->bm_positions, ix->bm_tomb.p, rs->bits.p, rs->nbits, 0, bw, rs->bm_mask.p, nullptr, s);
+        else
+            launch_rowset_mask(ix->d_members.p, ix->bm_positions, ix->bm_tomb.p, rs->bits.p, rs->nbits, 0, bw, rs->bm_mask.p, nullptr, s);
+    }
+    ZB_CUDA(cudaMemcpyAsync(&rs->n_live, rs->d_live.p, 8, cudaMemcpyDeviceToHost, s));
+    ix->sync();
+    rs->gen = ix->mut_gen;
+}
+
+// Gathers the rows the slot mask leaves in into the rowset's dense store, in slot order (= ordinal order), with the side
+// arrays of the exact search computed by the same kernels as over the raw store.
+static void rowset_compact(zb_index* ix, zb_rowset* rs) {
+    cudaStream_t s = ix->stream;
+    const u64 n = ix->n_slots, wn = (n + 31) / 32, c = rs->n_live, ca = c ? c : 1;
+    DBuf<u32> wl, woff;
+    wl.ensure(wn + 1);
+    woff.ensure(wn + 1);
+    ZB_CUDA(cudaMemsetAsync(wl.p + wn, 0, 4, s));
+    launch_rowset_word_live(rs->slot_mask.p, wn, wl.p, s);
+    ix->scan_tmp(wn + 1);
+    exclusive_scan_u32(ix->cub_tmp.p, ix->cub_tmp.bytes(), wl.p, woff.p, wn + 1, s);
+    rs->c_slot.ensure(ca);
+    rs->c_ord.ensure(ca);
+    rs->c_rows.ensure(ca * (u64)ix->dimp);
+    launch_rowset_compact(rs->slot_mask.p, n, woff.p, rs->c_slot.p, s);
+    // every gathered slot is clear in the slot mask, so the key written is the bare ordinal
+    launch_pack_rows(rs->c_slot.p, c, ix->rows.p, ix->ord.p, rs->slot_mask.p, ix->dimp, rs->c_rows.p, rs->c_ord.p, s);
+    if (ix->opt.metric == ZB_METRIC_COSINE) {
+        rs->c_rinv.ensure(ca);
+        launch_rinv(rs->c_rows.p, c, ix->dimp, rs->c_rinv.p, s);
+    } else {
+        rs->c_n2.ensure(ca);
+        launch_n2(rs->c_rows.p, c, ix->dimp, rs->c_n2.p, s);
+    }
+    rs->c_mask.ensure(c / 32 + 8);
+    ix->sync();
+    rs->c_n = c;
+    rs->c_gen = ~0ull;
+    rs->compact = true;
+}
 
 // nq = queries of the whole batch.  Unsharded, or sharded with sliced == false: d_q holds all of them and the outputs hold
 // all nq results (on every rank).  Sharded with sliced == true (the scalable form): d_q holds only the slice this rank
 // fronts, queries [rank * nqp, (rank + 1) * nqp) with nqp = ceil(nq / G); the slices are allgathered over NVLink into
 // q_all, and the outputs receive the results of the rank's own slice only (no result allgather).
 // probes > 0: multi-probe walk (DESIGN 3.9); the visits it appends go through the same compaction, scan and merge.
+// rs: restricted search (DESIGN 3.10): the rowset's masks and leaf counts replace the tombstones and live counts.
 static void search_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u32 probes, u64* d_out_ord, u64* d_out_bits,
-                          u32* d_out_counts, bool sliced) {
+                          u32* d_out_counts, bool sliced, zb_rowset* rs = nullptr) {
     cudaStream_t s = ix->stream;
     const u32 T = ix->T;
     ix->st.last_queries = nq;
@@ -1022,7 +1129,7 @@ static void search_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u32
     }
     if (sharded) ix->ensure_bucket_major();  // collective (rebuilds the bucket-sharded store after a forest change)
     ForestView f = ix->view();              // the plan walks the replicated forest with GLOBAL live leaf counts
-    const ForestView fs = ix->scan_view();  // scoring reads the leaves this rank holds
+    ForestView fs = ix->scan_view();        // scoring reads the leaves this rank holds
     const u64 nw = nqp * (sharded ? G : 1) * T;  // walkers, padded to G equal slices
     const u64 nwl = nqp * T;                     // walkers this rank plans
     ZB_REQUIRE(nw < (1ull << 31), ZB_ERR_INVALID, "batch too large: %llu walkers", (unsigned long long)nw);
@@ -1072,6 +1179,14 @@ static void search_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u32
     const bool gen3 = ix->p_scan_gen != 2 && tile_scan3_supported(ix->dimp, (u32)top_k);
     const bool tile_on = ix->opt.metric <= ZB_METRIC_L2 && ix->p_use_tile_scan && ix->opt.max_node_size >= (u64)ix->p_tile_min_rows &&
                          (gen3 || tile_scan_supported(ix->dimp, (u32)top_k)) && ix->ensure_bucket_major();
+    BucketMajor bmv = ix->bm_view();
+    if (rs) {
+        rowset_derive(ix, rs);
+        f.leaf_plan = fs.leaf_plan = sharded ? rs->leaf_plan.p : rs->leaf_live.p;
+        f.tomb = rs->slot_mask.p;
+        fs.tomb = sharded ? rs->bm_mask.p : rs->slot_mask.p;
+        bmv.tomb = rs->bm_mask.p;
+    }
     u64 v_cap = std::max<u64>(ix->v_leaf.cap ? ix->v_leaf.cap - 1 : 0, nw * (1 + (u64)probes) + nw / 2 + 1024);
     // a walker's region holds its cascade (31 visits by default) plus its probe visits, so the first probe batch needs no replan
     if (probes) ix->vpw = std::max<u32>(ix->vpw, 32 + probes);
@@ -1206,7 +1321,7 @@ static void search_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u32
         // last batches had to rescan too many visits exactly, 2 always)
         ix->scan_ws.l2_filter = gen3 && ix->dimp >= 128 && (ix->p_l2_filter == 2 || (ix->p_l2_filter == 1 && ix->filter_backoff == 0));
         if (ix->filter_backoff > 0) --ix->filter_backoff;
-        (gen3 ? tile_scan3 : tile_scan)(ix->scan_ws, fs, ix->bm_view(), ix->opt.metric, d_q, ix->q_rinv.p, (u32)nq, nv, ix->v_leaf.p,
+        (gen3 ? tile_scan3 : tile_scan)(ix->scan_ws, fs, bmv, ix->opt.metric, d_q, ix->q_rinv.p, (u32)nq, nv, ix->v_leaf.p,
                                         ix->v_np.p, ix->v_q.p, ix->v_ent_off.p, ix->v_pair_len.p, ix->v_done.p, ix->entries.p,
                                         (u32)top_k, (u32)ix->p_tile_min_rows, (u32)ix->p_tile_queries,
                                         (u32)ix->h_leaf_off.size(), s);
@@ -1332,7 +1447,11 @@ static void search_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u32
 // scans the rows it owns; a sharded call allgathers the ranks' per-query lists and merges them (the same exchange as the
 // unsliced search).  Queries go in chunks that keep the workspace within the exact_budget_mb knob; the plan comes from the
 // largest row count of all ranks, so every rank runs the same sequence of collectives.
-static void exact_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64* d_out_ord, u64* d_out_bits, u32* d_out_counts) {
+// rs: restricted exact search (DESIGN 3.10).  When the rows of the set live on this rank are at most half of its slots, they
+// are gathered once into the rowset's own dense store (ordinals ascending, so ties still break by ordinal) and scanned
+// there; otherwise the raw store is scanned with the rowset's slot mask.
+static void exact_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64* d_out_ord, u64* d_out_bits, u32* d_out_counts,
+                         zb_rowset* rs = nullptr) {
     cudaStream_t s = ix->stream;
     if (!nq) return;
     if (!top_k) {
@@ -1341,21 +1460,11 @@ static void exact_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64*
     }
     const u32 G = ix->G;
     const bool sharded = G > 1;
-    u64 n_max = ix->n_slots;
-    if (sharded) {
-        ix->ex_nmax.ensure(1);
-        ZB_CUDA(cudaMemcpyAsync(ix->ex_nmax.p, &n_max, 8, cudaMemcpyHostToDevice, s));
-        ix->nccl.allreduce(ix->ex_nmax.p, 1, Nccl::U64, Nccl::MAX, s);
-        ZB_CUDA(cudaMemcpyAsync(&n_max, ix->ex_nmax.p, 8, cudaMemcpyDeviceToHost, s));
-        ix->sync();
-    }
     const u32 metric = ix->opt.metric;
     // L2 / L2 squared with short lists go through the dot-product filter, as in the LSH search (DESIGN 3.8: measured on config 2)
     const bool filt = (metric == ZB_METRIC_L2SQ || metric == ZB_METRIC_L2) && top_k <= ZB_L2_FILTER_MAX_K && ix->dimp >= 128;
     ix->ensure_exact_side();
-    // per query: q_rinv / q_n2 / shared bound, and (sharded) its local lists plus the G gathered ones
-    const u64 per_query = 24 + (sharded ? 16 * top_k * (G + 1) + 4 : 0);
-    const ExactPlan p = exact_plan(n_max, nq, ix->dimp, (u32)top_k, filt, per_query, (u64)ix->p_exact_budget_mb << 20);
+    u64 n = ix->n_slots;
     ForestView store = ix->view();
     store.members = ix->ex_iota.p;
     BucketMajor bm;
@@ -1363,15 +1472,44 @@ static void exact_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64*
     bm.tomb = ix->tomb.p;
     bm.rinv = metric == ZB_METRIC_COSINE ? ix->ex_rinv.p : nullptr;
     bm.n2 = filt ? ix->ex_n2.p : nullptr;
+    if (rs) {
+        rowset_derive(ix, rs);
+        if (!rs->compact && rs->n_live * 2 <= ix->n_slots) rowset_compact(ix, rs);
+        if (rs->compact) {
+            if (rs->c_gen != rs->gen) {   // rows of the set removed since the gather
+                launch_rowset_mask(rs->c_slot.p, rs->c_n, nullptr, rs->slot_mask.p, ix->n_slots, 1, rs->c_n / 32 + 8, rs->c_mask.p, nullptr, s);
+                rs->c_gen = rs->gen;
+            }
+            n = rs->c_n;
+            store.rows = bm.rows = rs->c_rows.p;
+            store.ord = rs->c_ord.p;
+            store.tomb = bm.tomb = rs->c_mask.p;
+            bm.rinv = metric == ZB_METRIC_COSINE ? rs->c_rinv.p : nullptr;
+            bm.n2 = filt ? rs->c_n2.p : nullptr;
+        } else {
+            store.tomb = bm.tomb = rs->slot_mask.p;
+        }
+    }
+    u64 n_max = n;
+    if (sharded) {
+        ix->ex_nmax.ensure(1);
+        ZB_CUDA(cudaMemcpyAsync(ix->ex_nmax.p, &n_max, 8, cudaMemcpyHostToDevice, s));
+        ix->nccl.allreduce(ix->ex_nmax.p, 1, Nccl::U64, Nccl::MAX, s);
+        ZB_CUDA(cudaMemcpyAsync(&n_max, ix->ex_nmax.p, 8, cudaMemcpyDeviceToHost, s));
+        ix->sync();
+    }
+    // per query: q_rinv / q_n2 / shared bound, and (sharded) its local lists plus the G gathered ones
+    const u64 per_query = 24 + (sharded ? 16 * top_k * (G + 1) + 4 : 0);
+    const ExactPlan p = exact_plan(n_max, nq, ix->dimp, (u32)top_k, filt, per_query, (u64)ix->p_exact_budget_mb << 20);
     alignas(64) unsigned char tmap[128];
-    if (ix->n_slots) make_row_tile_map(tmap, ix->rows.p, ix->n_slots, ix->dimp, 64, tile_scan_box_floats(3));
+    if (n) make_row_tile_map(tmap, bm.rows, n, ix->dimp, 64, tile_scan_box_floats(3));
     bm.tmap3 = tmap;
-    bm.positions = ix->n_slots;
+    bm.positions = n;
     for (u64 c0 = 0; c0 < nq; c0 += p.chunk) {
         const u64 c = std::min<u64>(p.chunk, nq - c0);
         const float* q = d_q + c0 * (u64)ix->dimp;
         if (!sharded) {
-            exact_scan3(ix->ex_ws, store, bm, ix->n_slots, metric, q, (u32)c, p.range_rows, (u32)top_k, filt, d_out_ord + c0 * top_k,
+            exact_scan3(ix->ex_ws, store, bm, n, metric, q, (u32)c, p.range_rows, (u32)top_k, filt, d_out_ord + c0 * top_k,
                         d_out_bits + c0 * top_k, d_out_counts + c0, s);
             continue;
         }
@@ -1379,7 +1517,7 @@ static void exact_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u64*
         ix->ex_loc.ensure(2 * p.chunk * top_k);
         ix->ex_gath.ensure(2 * p.chunk * top_k * G);
         ix->ex_counts.ensure(p.chunk);
-        exact_scan3(ix->ex_ws, store, bm, ix->n_slots, metric, q, (u32)c, p.range_rows, (u32)top_k, filt, ix->ex_loc.p,
+        exact_scan3(ix->ex_ws, store, bm, n, metric, q, (u32)c, p.range_rows, (u32)top_k, filt, ix->ex_loc.p,
                     ix->ex_loc.p + nsk, ix->ex_counts.p, s);
         ix->nccl.allgather(ix->ex_loc.p, ix->ex_gath.p, 2 * nsk * 8, s);
         launch_merge_gathered((u32)c, (u32)c, (u32)top_k, G, ix->ex_gath.p, d_out_ord + c0 * top_k, d_out_bits + c0 * top_k,
@@ -1646,6 +1784,7 @@ static void remove_ordinals(zb_index* ix, u64 n, const u64* ordinals, const u8* 
         ZB_CUDA(cudaMemcpyAsync(flags.data(), ix->rm_flags.p, n, cudaMemcpyDeviceToHost, ix->stream));
     }
     ix->refresh_plan_counts();
+    ++ix->mut_gen;
     ix->sync();
     for (u64 i = 0; i < n; ++i) {
         if (flags[i] && slots[i] != 0xFFFFFFFFu && !ix->h_tomb[slots[i]]) {
@@ -1818,7 +1957,7 @@ int zb_index_no_trees(zb_index* ix, int* out) {
 // Batches beyond 131072 queries are cut into chunks (walker count < 2^31, bounded workspaces).  sliced: see search_device;
 // the chunks of a sliced call are chunks of the whole batch, so every rank sees the same sequence of collectives.
 static void search_entry_device(zb_index* ix, u64 nq, const float* d_q, u64 top_k, u32 probes, u64* d_out_ord, u64* d_out_bits,
-                                u32* d_out_counts, bool sliced, bool exact = false) {
+                                u32* d_out_counts, bool sliced, bool exact = false, zb_rowset* rs = nullptr) {
     ix->use_device();
     const u64 G = ix->G;
     sliced = sliced && G > 1;
@@ -1832,8 +1971,8 @@ static void search_entry_device(zb_index* ix, u64 nq, const float* d_q, u64 top_
             mine = std::min<u64>(nqp, c - lo);
         }
         const float* q = stage_queries_device(ix, d_q + in_off * (u64)ix->dim, mine);
-        if (exact) exact_device(ix, c, q, top_k, d_out_ord + in_off * top_k, d_out_bits + in_off * top_k, d_out_counts + in_off);
-        else search_device(ix, c, q, top_k, probes, d_out_ord + in_off * top_k, d_out_bits + in_off * top_k, d_out_counts + in_off, sliced);
+        if (exact) exact_device(ix, c, q, top_k, d_out_ord + in_off * top_k, d_out_bits + in_off * top_k, d_out_counts + in_off, rs);
+        else search_device(ix, c, q, top_k, probes, d_out_ord + in_off * top_k, d_out_bits + in_off * top_k, d_out_counts + in_off, sliced, rs);
         in_off += mine;
     }
     ix->sync();
@@ -1860,7 +1999,8 @@ int zb_index_search_slice_device(zb_index* ix, uint64_t nq_total, const float* d
 
 // Host buffers in, host buffers out.  sliced: `queries` and the outputs hold this rank's slices only.
 static void search_entry_host(zb_index* ix, u64 nq, const float* queries, u64 top_k, u32 probes, uint8_t* out_ids16,
-                              u64* out_ordinals, u64* out_bits, u32* out_counts, bool sliced, bool exact = false) {
+                              u64* out_ordinals, u64* out_bits, u32* out_counts, bool sliced, bool exact = false,
+                              zb_rowset* rs = nullptr) {
     ix->use_device();
     cudaStream_t s = ix->stream;
     const u64 G = ix->G;
@@ -1900,8 +2040,8 @@ static void search_entry_host(zb_index* ix, u64 nq, const float* queries, u64 to
         ix->o_ord.ensure(mine * top_k + 1);
         ix->o_bits.ensure(mine * top_k + 1);
         ix->o_counts2.ensure(mine + 1);
-        if (exact) exact_device(ix, c, ix->q_stage.p, top_k, ix->o_ord.p, ix->o_bits.p, ix->o_counts2.p);
-        else search_device(ix, c, ix->q_stage.p, top_k, probes, ix->o_ord.p, ix->o_bits.p, ix->o_counts2.p, sliced);
+        if (exact) exact_device(ix, c, ix->q_stage.p, top_k, ix->o_ord.p, ix->o_bits.p, ix->o_counts2.p, rs);
+        else search_device(ix, c, ix->q_stage.p, top_k, probes, ix->o_ord.p, ix->o_bits.p, ix->o_counts2.p, sliced, rs);
         if (!out_ordinals && out_ids16) ord_tmp.resize(mine * top_k);
         u64* ords = out_ordinals ? out_ordinals + in_off * top_k : ord_tmp.data();
         if (top_k && mine) {
@@ -2042,6 +2182,155 @@ int zb_index_search_slice_probe_device(zb_index* ix, uint64_t nq_total, const fl
     probe_check(top_k, probes);
     std::lock_guard<std::mutex> lk(ix->mu);
     search_entry_device(ix, nq_total, d_q, top_k, probes, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, true);
+    ZB_API_END
+}
+
+// ---------------------------------------------------------------- rowsets / restricted search (DESIGN 3.10)
+// h_ords (host, already checked < total_rows) or d_ords (device, checked by the scatter kernel): the listed ordinals.
+static zb_rowset* rowset_make(zb_index* ix, u64 n, const u64* h_ords, const u64* d_ords, uint32_t flags) {
+    ZB_REQUIRE(!(flags & ~(uint32_t)ZB_ROWSET_EXCLUDE), ZB_ERR_INVALID, "rowset flags 0x%x: only ZB_ROWSET_EXCLUDE is defined", flags);
+    ix->use_device();
+    cudaStream_t s = ix->stream;
+    std::unique_ptr<zb_rowset> rs(new zb_rowset());
+    rs->ix = ix;
+    rs->epoch = ix->content_epoch;
+    rs->nbits = ix->total_rows;
+    const u64 words = rs->nbits / 32 + 1;
+    rs->bits.ensure(words);
+    rs->d_live.ensure(2);   // [0] the set's size, [1] the unknown-ordinal flag
+    ZB_CUDA(cudaMemsetAsync(rs->bits.p, 0, words * 4, s));
+    ZB_CUDA(cudaMemsetAsync(rs->d_live.p, 0, 16, s));
+    DBuf<u64> up;
+    if (h_ords && n) {
+        up.ensure(n);
+        ZB_CUDA(cudaMemcpyAsync(up.p, h_ords, n * 8, cudaMemcpyHostToDevice, s));
+        d_ords = up.p;
+    }
+    launch_rowset_scatter(d_ords, n, rs->nbits, rs->bits.p, reinterpret_cast<u32*>(rs->d_live.p + 1), s);
+    launch_rowset_finish(rs->bits.p, rs->nbits, words, (flags & ZB_ROWSET_EXCLUDE) ? 1u : 0u, rs->d_live.p, s);
+    u64 h[2] = {0, 0};
+    ZB_CUDA(cudaMemcpyAsync(h, rs->d_live.p, 16, cudaMemcpyDeviceToHost, s));
+    ix->sync();
+    ZB_REQUIRE(!h[1], ZB_ERR_INVALID, "rowset: an ordinal is >= the %llu rows of the index", (unsigned long long)rs->nbits);
+    rs->count = h[0];
+    return rs.release();
+}
+
+int zb_index_rowset_from_ordinals(zb_index* ix, uint64_t n, const uint64_t* ordinals, uint32_t flags, uint64_t* out_count,
+                                  zb_rowset** out) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && out && (ordinals || !n), ZB_ERR_INVALID, "NULL argument");
+    *out = nullptr;
+    std::lock_guard<std::mutex> lk(ix->mu);
+    for (u64 i = 0; i < n; ++i)
+        ZB_REQUIRE(ordinals[i] < ix->total_rows, ZB_ERR_INVALID, "rowset: ordinal %llu at %llu is >= the %llu rows of the index",
+                   (unsigned long long)ordinals[i], (unsigned long long)i, (unsigned long long)ix->total_rows);
+    zb_rowset* rs = rowset_make(ix, n, (const u64*)ordinals, nullptr, flags);
+    if (out_count) *out_count = rs->count;
+    *out = rs;
+    ZB_API_END
+}
+int zb_index_rowset_from_ordinals_device(zb_index* ix, uint64_t n, const uint64_t* d_ordinals, uint32_t flags, uint64_t* out_count,
+                                         zb_rowset** out) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && out && (d_ordinals || !n), ZB_ERR_INVALID, "NULL argument");
+    *out = nullptr;
+    std::lock_guard<std::mutex> lk(ix->mu);
+    zb_rowset* rs = rowset_make(ix, n, nullptr, (const u64*)d_ordinals, flags);
+    if (out_count) *out_count = rs->count;
+    *out = rs;
+    ZB_API_END
+}
+int zb_index_rowset_from_ids(zb_index* ix, uint64_t n, const uint8_t* ids16, uint32_t flags, uint8_t* out_found, uint64_t* out_count,
+                             zb_rowset** out) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && out && (ids16 || !n), ZB_ERR_INVALID, "NULL argument");
+    *out = nullptr;
+    std::lock_guard<std::mutex> lk(ix->mu);
+    std::vector<u64> ords;
+    ords.reserve(n);
+    for (u64 i = 0; i < n; ++i) {
+        u64 o = 0;
+        const bool found = ix->ordinal_of(ids16 + 16 * i, &o);
+        if (found) ords.push_back(o);
+        if (out_found) out_found[i] = found ? 1 : 0;
+    }
+    zb_rowset* rs = rowset_make(ix, ords.size(), ords.data(), nullptr, flags);
+    if (out_count) *out_count = rs->count;
+    *out = rs;
+    ZB_API_END
+}
+int zb_rowset_destroy(zb_rowset* rs) {
+    ZB_API_BEGIN
+    if (!rs) return ZB_OK;
+    {
+        std::lock_guard<std::mutex> lk(rs->ix->mu);
+        rs->ix->use_device();
+        rs->ix->sync();
+        delete rs;
+    }
+    ZB_API_END
+}
+
+int zb_index_search_rowset(zb_index* ix, uint64_t nq, const float* queries, uint64_t top_k, uint32_t probes, zb_rowset* rowset,
+                           uint8_t* out_ids16, uint64_t* out_ordinals, uint64_t* out_bits, uint32_t* out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && (queries || !nq) && ((out_bits && out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
+    probe_check(top_k, probes);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    if (rowset) rowset_check(ix, rowset);
+    search_entry_host(ix, nq, queries, top_k, probes, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, false, false, rowset);
+    ZB_API_END
+}
+int zb_index_search_rowset_device(zb_index* ix, uint64_t nq, const float* d_q, uint64_t top_k, uint32_t probes, zb_rowset* rowset,
+                                  uint64_t* d_out_ord, uint64_t* d_out_bits, uint32_t* d_out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && (d_q || !nq) && ((d_out_ord && d_out_bits && d_out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
+    probe_check(top_k, probes);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    if (rowset) rowset_check(ix, rowset);
+    search_entry_device(ix, nq, d_q, top_k, probes, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, false, false, rowset);
+    ZB_API_END
+}
+int zb_index_search_slice_rowset(zb_index* ix, uint64_t nq_total, const float* queries, uint64_t top_k, uint32_t probes,
+                                 zb_rowset* rowset, uint8_t* out_ids16, uint64_t* out_ordinals, uint64_t* out_bits,
+                                 uint32_t* out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix, ZB_ERR_INVALID, "NULL argument");
+    probe_check(top_k, probes);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    if (rowset) rowset_check(ix, rowset);
+    search_entry_host(ix, nq_total, queries, top_k, probes, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, true, false, rowset);
+    ZB_API_END
+}
+int zb_index_search_slice_rowset_device(zb_index* ix, uint64_t nq_total, const float* d_q, uint64_t top_k, uint32_t probes,
+                                        zb_rowset* rowset, uint64_t* d_out_ord, uint64_t* d_out_bits, uint32_t* d_out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix, ZB_ERR_INVALID, "NULL argument");
+    probe_check(top_k, probes);
+    std::lock_guard<std::mutex> lk(ix->mu);
+    if (rowset) rowset_check(ix, rowset);
+    search_entry_device(ix, nq_total, d_q, top_k, probes, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, true, false, rowset);
+    ZB_API_END
+}
+int zb_index_search_exact_rowset(zb_index* ix, uint64_t nq, const float* queries, uint64_t top_k, zb_rowset* rowset, uint8_t* out_ids16,
+                                 uint64_t* out_ordinals, uint64_t* out_bits, uint32_t* out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && (queries || !nq) && ((out_bits && out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
+    std::lock_guard<std::mutex> lk(ix->mu);
+    exact_check(ix, top_k);
+    if (rowset) rowset_check(ix, rowset);
+    search_entry_host(ix, nq, queries, top_k, 0, out_ids16, (u64*)out_ordinals, (u64*)out_bits, out_counts, false, true, rowset);
+    ZB_API_END
+}
+int zb_index_search_exact_rowset_device(zb_index* ix, uint64_t nq, const float* d_q, uint64_t top_k, zb_rowset* rowset,
+                                        uint64_t* d_out_ord, uint64_t* d_out_bits, uint32_t* d_out_counts) {
+    ZB_API_BEGIN
+    ZB_REQUIRE(ix && (d_q || !nq) && ((d_out_ord && d_out_bits && d_out_counts) || !nq), ZB_ERR_INVALID, "NULL argument");
+    std::lock_guard<std::mutex> lk(ix->mu);
+    exact_check(ix, top_k);
+    if (rowset) rowset_check(ix, rowset);
+    search_entry_device(ix, nq, d_q, top_k, 0, (u64*)d_out_ord, (u64*)d_out_bits, d_out_counts, false, true, rowset);
     ZB_API_END
 }
 
@@ -2191,6 +2480,8 @@ static void clear_locked(zb_index* ix) {
     ix->clear_forest();
     ix->n_slots = ix->n_live = ix->total_rows = 0;
     ++ix->store_gen;
+    ++ix->mut_gen;
+    ++ix->content_epoch;
     ix->h_ord.clear();
     ix->h_tomb.clear();
     ix->flat_bits = 0;

@@ -1762,6 +1762,92 @@ size_t maxscan_temp_bytes(size_t n) {
 }
 
 // =====================================================================================================
+// rowsets (restricted search, DESIGN 3.10): a bitmap over global ordinals, and the masks a restricted search substitutes
+// for the tombstones
+// =====================================================================================================
+__global__ void rowset_scatter_kernel(const u64* __restrict__ ords, u64 n, u64 nbits, u32* __restrict__ bits, u32* __restrict__ bad) {
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const u64 o = ords[i];
+    if (o >= nbits) {
+        atomicOr(bad, 1u);
+        return;
+    }
+    atomicOr(&bits[o >> 5], 1u << (o & 31));
+}
+void launch_rowset_scatter(const u64* d_ords, u64 n, u64 nbits, u32* d_bits, u32* d_bad, cudaStream_t s) {
+    if (!n) return;
+    rowset_scatter_kernel<<<(u32)((n + 255) / 256), 256, 0, s>>>(d_ords, n, nbits, d_bits, d_bad);
+}
+// exclude mode: complement over [0, nbits); bits at or above nbits are cleared either way; count += members of the set
+__global__ void rowset_finish_kernel(u32* __restrict__ bits, u64 nbits, u64 words, u32 invert, u64* __restrict__ count) {
+    const u64 w = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    u32 c = 0;
+    if (w < words) {
+        u32 v = invert ? ~bits[w] : bits[w];
+        const u64 lo = w * 32;
+        if (lo >= nbits) v = 0;
+        else if (nbits - lo < 32) v &= (1u << (nbits - lo)) - 1u;
+        bits[w] = v;
+        c = __popc(v);
+    }
+    c = __reduce_add_sync(0xFFFFFFFFu, c);
+    if ((threadIdx.x & 31) == 0 && c) atomicAdd(count, (u64)c);
+}
+void launch_rowset_finish(u32* d_bits, u64 nbits, u64 words, u32 invert, u64* d_count, cudaStream_t s) {
+    if (!words) return;
+    rowset_finish_kernel<<<(u32)((words + 255) / 256), 256, 0, s>>>(d_bits, nbits, words, invert, d_count);
+}
+// out bit p (p < 32 * words) = removed for a restricted search: p >= n, or own bit p set (the tombstones, when given), or the
+// bit of key[p] in `bits` says so (bits_dead = 0: `bits` is the rowset, a clear or out-of-range bit excludes; bits_dead = 1:
+// `bits` is a mask of removed positions).  live += positions left in.
+template <class K>
+__global__ void rowset_mask_kernel(const K* __restrict__ key, u64 n, const u32* __restrict__ own, const u32* __restrict__ bits,
+                                   u64 nbits, u32 bits_dead, u64 words, u32* __restrict__ out, u64* __restrict__ live) {
+    const u64 p = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    bool dead = true;
+    if (p < n) {
+        const u64 k = key[p];
+        const bool b = k < nbits && ((bits[k >> 5] >> (k & 31)) & 1u);
+        dead = (own && tomb_test(own, (u32)p)) || (b == (bits_dead != 0));
+    }
+    const u32 w = __ballot_sync(0xFFFFFFFFu, dead);
+    if ((threadIdx.x & 31) == 0 && (p >> 5) < words) {
+        out[p >> 5] = w;
+        if (live && ~w) atomicAdd(live, (u64)__popc(~w));
+    }
+}
+void launch_rowset_mask(const u64* d_key, u64 n, const u32* d_own, const u32* d_bits, u64 nbits, u32 bits_dead, u64 words, u32* d_out,
+                        u64* d_live, cudaStream_t s) {
+    if (!words) return;
+    rowset_mask_kernel<u64><<<(u32)((words * 32 + 255) / 256), 256, 0, s>>>(d_key, n, d_own, d_bits, nbits, bits_dead, words, d_out, d_live);
+}
+void launch_rowset_mask(const u32* d_key, u64 n, const u32* d_own, const u32* d_bits, u64 nbits, u32 bits_dead, u64 words, u32* d_out,
+                        u64* d_live, cudaStream_t s) {
+    if (!words) return;
+    rowset_mask_kernel<u32><<<(u32)((words * 32 + 255) / 256), 256, 0, s>>>(d_key, n, d_own, d_bits, nbits, bits_dead, words, d_out, d_live);
+}
+// compaction of the positions a mask leaves in, ascending: per-word counts, (exclusive scan), then every position's rank
+__global__ void rowset_word_live_kernel(const u32* __restrict__ mask, u64 words, u32* __restrict__ out) {
+    const u64 w = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (w < words) out[w] = __popc(~mask[w]);
+}
+void launch_rowset_word_live(const u32* d_mask, u64 words, u32* d_out, cudaStream_t s) {
+    if (!words) return;
+    rowset_word_live_kernel<<<(u32)((words + 255) / 256), 256, 0, s>>>(d_mask, words, d_out);
+}
+__global__ void rowset_compact_kernel(const u32* __restrict__ mask, u64 n, const u32* __restrict__ woff, u32* __restrict__ out) {
+    const u64 p = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n) return;
+    const u32 m = ~mask[p >> 5], b = (u32)(p & 31);
+    if ((m >> b) & 1u) out[woff[p >> 5] + __popc(m & ((1u << b) - 1u))] = (u32)p;
+}
+void launch_rowset_compact(const u32* d_mask, u64 n, const u32* d_woff, u32* d_out, cudaStream_t s) {
+    if (!n) return;
+    rowset_compact_kernel<<<(u32)((n + 255) / 256), 256, 0, s>>>(d_mask, n, d_woff, d_out);
+}
+
+// =====================================================================================================
 // cub scans / sorts
 // =====================================================================================================
 size_t scan_temp_bytes(size_t n) {

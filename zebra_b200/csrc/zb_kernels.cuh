@@ -134,6 +134,21 @@ size_t sort_temp_bytes(size_t n);
 void sort_pairs_u64_u32(void* d_temp, size_t temp_bytes, const u64* d_kin, u64* d_kout, const u32* d_vin, u32* d_vout, size_t n,
                         int end_bit, cudaStream_t s);
 
+// ---- rowsets (restricted search, DESIGN 3.10) ----
+// bits[o / 32] |= 1 << o % 32 for every listed ordinal; *bad = 1 if one is >= nbits
+void launch_rowset_scatter(const u64* d_ords, u64 n, u64 nbits, u32* d_bits, u32* d_bad, cudaStream_t s);
+// invert (exclude mode) over [0, nbits), clear the bits at or above nbits, *count += the set's size
+void launch_rowset_finish(u32* d_bits, u64 nbits, u64 words, u32 invert, u64* d_count, cudaStream_t s);
+// out[0, words): bit p set = position p is removed for a restricted search (p >= n, tombstone bit p of d_own if given, or
+// the bit of key[p] in d_bits: clear for bits_dead = 0, set for bits_dead = 1); *d_live += positions left in (if given)
+void launch_rowset_mask(const u64* d_key, u64 n, const u32* d_own, const u32* d_bits, u64 nbits, u32 bits_dead, u64 words, u32* d_out,
+                        u64* d_live, cudaStream_t s);
+void launch_rowset_mask(const u32* d_key, u64 n, const u32* d_own, const u32* d_bits, u64 nbits, u32 bits_dead, u64 words, u32* d_out,
+                        u64* d_live, cudaStream_t s);
+// ascending list of the positions a mask leaves in: per-word counts -> exclusive scan (d_woff) -> positions
+void launch_rowset_word_live(const u32* d_mask, u64 words, u32* d_out, cudaStream_t s);
+void launch_rowset_compact(const u32* d_mask, u64 n, const u32* d_woff, u32* d_out, cudaStream_t s);
+
 // ---- deduplicate (lsh.rs:270-288) ----
 void launch_row_hash(const u32* d_slots, u64 n, const float* d_rows, int dimp, u64* d_h1, u64* d_h2, cudaStream_t s);
 void launch_dup_mark(const u64* d_sorted_key, const u32* d_cand, u64 n, const u32* d_slots, const float* d_rows, int dimp,

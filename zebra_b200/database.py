@@ -13,7 +13,7 @@ from typing import Dict, List, Optional, Sequence
 import numpy as np
 
 from .distance import CosineDistance, _DeviceMetric
-from .index import LSHIndex, LSHIndexOptions, _bytes_to_ids
+from .index import LSHIndex, LSHIndexOptions, RowSet, _bytes_to_ids
 
 
 class DatabaseEmbeddingModel:
@@ -103,12 +103,19 @@ class Database:
             return {}
         return self.query_vectors(self.model.embed_documents(documents), number_of_results)
 
-    def query_vectors(self, vectors, number_of_results: int, probes: int = 0) -> Dict[int, Dict[_uuid.UUID, bytes]]:  # core.rs:290-313
-        """probes > 0: multi-probe search (LSHIndex.search_batch); 0 is the reference's query."""
+    def query_vectors(self, vectors, number_of_results: int, probes: int = 0,
+                      within=None) -> Dict[int, Dict[_uuid.UUID, bytes]]:  # core.rs:290-313
+        """probes > 0: multi-probe search (LSHIndex.search_batch); 0 is the reference's query.  within: a RowSet of
+        `self.index`, or an iterable of document ids (unknown ids are ignored); only those documents are searched, as if
+        every other one had been removed (restricted search, DESIGN 3.10)."""
         if self.index.no_vectors():
             return {}
         vectors = np.ascontiguousarray(vectors, dtype=np.float32).reshape(-1, self.dim)
-        ids, _, _, counts = self.index.search_batch(vectors, number_of_results, probes=probes)  # ONE batched device call
+        if within is not None and not isinstance(within, RowSet):
+            with self.index.rowset(ids=within) as rs:
+                return self.query_vectors(vectors, number_of_results, probes, rs)
+        ids, _, _, counts = self.index.search_batch(vectors, number_of_results, probes=probes,
+                                                    within=within)  # ONE batched device call
         out: Dict[int, Dict[_uuid.UUID, bytes]] = {}
         for q in range(vectors.shape[0]):
             out[q] = {i: self._documents.get(i, b"") for i in _bytes_to_ids(ids[q, : int(counts[q])])}

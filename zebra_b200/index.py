@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import uuid as _uuid
+import weakref
 from dataclasses import dataclass
 from typing import Iterable, List, Optional, Sequence, Set, Tuple
 
@@ -47,6 +48,45 @@ def _bytes_to_ids(raw: np.ndarray) -> List[_uuid.UUID]:
     return [_uuid.UUID(bytes=b[i:i + 16]) for i in range(0, len(b), 16)]
 
 
+ROWSET_EXCLUDE = 1  # ZB_ROWSET_EXCLUDE
+
+
+class RowSet:
+    """A fixed set of rows of one LSHIndex, for restricted search (`within=` of every search form, DESIGN 3.10).
+
+    Made by `LSHIndex.rowset`.  A restricted search returns exactly what the plain search would return if every live row
+    outside the set had been removed, without changing the index for anyone else.  The set is fixed when it is made: rows
+    added later are never in it; rows removed later are excluded at call time; inserts, leaf splits and deduplicate are
+    taken into account.  After `clear`, `load_forest`, `load_flat` or `import_store` (which reuse ordinals) a search with it
+    raises ZebraError (ZB_ERR_STATE).  It holds device memory: `close()` it, or use it as a context manager.  It keeps its
+    index alive; closing the index closes its rowsets.
+
+    `count`: ordinals in the set.  `found`: for a set made from ids, which ids the index knows (unknown ones are ignored)."""
+
+    def __init__(self, index: "LSHIndex", handle: C.c_void_p, count: int, found: Optional[np.ndarray] = None):
+        self.index = index
+        self._h = handle
+        self.count = count
+        self.found = found
+
+    def close(self) -> None:
+        if getattr(self, "_h", None) and self._h.value:
+            _ffi.check(_ffi.lib().zb_rowset_destroy(self._h))
+            self._h = C.c_void_p()
+
+    def __enter__(self) -> "RowSet":
+        return self
+
+    def __exit__(self, *exc) -> None:
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 class LSHIndex:
     """lsh.rs:145-148.  `metric` fixes the distance the device index scores with (the reference passes the
     metric to search(); a device index is built for ONE metric of distance.rs -- the fused leaf-tile scan serves
@@ -69,6 +109,7 @@ class LSHIndex:
         o.device, o.seed = device, seed
         o.shard_rank, o.shard_count = shard_rank, shard_count
         self._h = C.c_void_p()
+        self._rowsets = weakref.WeakSet()
         _ffi.check(_ffi.lib().zb_index_create(C.byref(o), C.byref(self._h)))
 
     # lsh.rs:162
@@ -78,6 +119,8 @@ class LSHIndex:
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:
+            for rs in list(getattr(self, "_rowsets", ())):  # a rowset belongs to its index: it goes first
+                rs.close()
             _ffi.lib().zb_index_destroy(self._h)
             self._h = C.c_void_p()
 
@@ -165,16 +208,51 @@ class LSHIndex:
         return self.no_vectors() or self.no_trees()
 
     # ---------------------------------------------------------------- lsh.rs:544-565
+    # ---------------------------------------------------------------- restricted search (DESIGN 3.10)
+    def rowset(self, ids: Optional[Sequence] = None, ordinals=None, exclude: bool = False) -> RowSet:
+        """The rows given by `ids` or by `ordinals` (one of the two; duplicates allowed), or with exclude=True every row
+        present now except those.  An ordinal at or beyond total_rows raises ZebraError; unknown ids are ignored and reported
+        in the RowSet's `found`.  Sharded index: every rank makes it from the same list."""
+        if (ids is None) == (ordinals is None):
+            raise ValueError("give ids or ordinals")
+        flags = ROWSET_EXCLUDE if exclude else 0
+        h, count, found = C.c_void_p(), C.c_uint64(), None
+        if ids is not None:
+            ids = list(ids)
+            idb = _ids_to_bytes(ids)
+            found = np.zeros(len(ids), dtype=np.uint8)
+            _ffi.check(_ffi.lib().zb_index_rowset_from_ids(self._h, len(ids), idb.ctypes.data if ids else None, flags,
+                                                           found.ctypes.data, C.byref(count), C.byref(h)))
+            found = found.astype(bool)
+        else:
+            o = np.ascontiguousarray(ordinals, dtype=np.uint64).reshape(-1)
+            _ffi.check(_ffi.lib().zb_index_rowset_from_ordinals(self._h, o.size, o.ctypes.data if o.size else None, flags,
+                                                                C.byref(count), C.byref(h)))
+        rs = RowSet(self, h, int(count.value), found)
+        self._rowsets.add(rs)
+        return rs
+
+    def _within(self, within: Optional[RowSet]):
+        if not isinstance(within, RowSet):
+            raise TypeError("within must be a RowSet made by LSHIndex.rowset")
+        if within.index is not self:
+            raise ValueError("within is a rowset of another index")
+        if not within._h.value:   # NULL would be the unrestricted search: a closed set must not widen it
+            raise ValueError("within is a closed RowSet")
+        return within._h
+
     # probes (every search form): 0 = the reference's search; P > 0 also visits, in every tree, the leaves across the P
     # main-path planes closest to the query (multi-probe, DESIGN 3.9; at most ZB_MAX_PROBES = 32)
-    def search(self, query, top_k: int, metric: Optional[_DeviceMetric] = None, probes: int = 0) -> List[Tuple[_uuid.UUID, int]]:
+    # within (every search form): a RowSet; the search runs as if every live row outside it had been removed (DESIGN 3.10)
+    def search(self, query, top_k: int, metric: Optional[_DeviceMetric] = None, probes: int = 0,
+               within: Optional[RowSet] = None) -> List[Tuple[_uuid.UUID, int]]:
         if metric is not None and metric != self.metric:
             raise ValueError("this device index was created for " + type(self.metric).__name__)
-        ids, _, bits, counts = self.search_batch(np.asarray(query, np.float32)[None, :], top_k, probes=probes)
+        ids, _, bits, counts = self.search_batch(np.asarray(query, np.float32)[None, :], top_k, probes=probes, within=within)
         c = int(counts[0])
         return list(zip(_bytes_to_ids(ids[0, :c]), (int(b) for b in bits[0, :c])))
 
-    def search_batch(self, queries, top_k: int, want_ids: bool = True, probes: int = 0):
+    def search_batch(self, queries, top_k: int, want_ids: bool = True, probes: int = 0, within: Optional[RowSet] = None):
         """One call for the whole batch (replaces the par_iter of core.rs:299).  Returns
         (ids [nq,k,16] uint8 or None, ordinals [nq,k] uint64, distance bits [nq,k] uint64, counts [nq] uint32)."""
         q = np.ascontiguousarray(queries, dtype=np.float32).reshape(-1, self.dim)
@@ -184,33 +262,39 @@ class LSHIndex:
         bits = np.empty((nq, top_k), dtype=np.uint64)
         counts = np.zeros(nq, dtype=np.uint32)
         self.search_batch_ptr(nq, q.ctypes.data, top_k, ords.ctypes.data, bits.ctypes.data, counts.ctypes.data,
-                              ids.ctypes.data if want_ids else None, probes=probes)
+                              ids.ctypes.data if want_ids else None, probes=probes, within=within)
         return ids, ords, bits, counts
 
     def search_batch_ptr(self, nq: int, q_ptr: int, top_k: int, ord_ptr: int, bits_ptr: int, counts_ptr: int,
-                         ids_ptr: Optional[int] = None, probes: int = 0) -> None:
+                         ids_ptr: Optional[int] = None, probes: int = 0, within: Optional[RowSet] = None) -> None:
         """Host-pointer form (e.g. pinned buffers owned by the caller)."""
-        if probes:
+        if within is not None:
+            _ffi.check(_ffi.lib().zb_index_search_rowset(self._h, nq, q_ptr, top_k, probes, self._within(within), ids_ptr, ord_ptr,
+                                                         bits_ptr, counts_ptr))
+        elif probes:
             _ffi.check(_ffi.lib().zb_index_search_probe(self._h, nq, q_ptr, top_k, probes, ids_ptr, ord_ptr, bits_ptr, counts_ptr))
         else:
             _ffi.check(_ffi.lib().zb_index_search_batch(self._h, nq, q_ptr, top_k, ids_ptr, ord_ptr, bits_ptr, counts_ptr))
 
     def search_batch_device(self, nq: int, d_q_ptr: int, top_k: int, d_ord_ptr: int, d_bits_ptr: int, d_counts_ptr: int,
-                            probes: int = 0):
-        if probes:
+                            probes: int = 0, within: Optional[RowSet] = None):
+        if within is not None:
+            _ffi.check(_ffi.lib().zb_index_search_rowset_device(self._h, nq, d_q_ptr, top_k, probes, self._within(within), d_ord_ptr,
+                                                                d_bits_ptr, d_counts_ptr))
+        elif probes:
             _ffi.check(_ffi.lib().zb_index_search_probe_device(self._h, nq, d_q_ptr, top_k, probes, d_ord_ptr, d_bits_ptr,
                                                                d_counts_ptr))
         else:
             _ffi.check(_ffi.lib().zb_index_search_batch_device(self._h, nq, d_q_ptr, top_k, d_ord_ptr, d_bits_ptr, d_counts_ptr))
 
     # ---------------------------------------------------------------- exact (brute-force) search, zb_index_search_exact
-    def search_exact(self, query, top_k: int) -> List[Tuple[_uuid.UUID, int]]:
-        """The true top_k over every live row, ordered like `search` (ground truth for its recall)."""
-        ids, _, bits, counts = self.search_exact_batch(np.asarray(query, np.float32)[None, :], top_k)
+    def search_exact(self, query, top_k: int, within: Optional[RowSet] = None) -> List[Tuple[_uuid.UUID, int]]:
+        """The true top_k over every live row (of `within`, if given), ordered like `search` (ground truth for its recall)."""
+        ids, _, bits, counts = self.search_exact_batch(np.asarray(query, np.float32)[None, :], top_k, within=within)
         c = int(counts[0])
         return list(zip(_bytes_to_ids(ids[0, :c]), (int(b) for b in bits[0, :c])))
 
-    def search_exact_batch(self, queries, top_k: int, want_ids: bool = True):
+    def search_exact_batch(self, queries, top_k: int, want_ids: bool = True, within: Optional[RowSet] = None):
         """Returns (ids [nq,k,16] uint8 or None, ordinals [nq,k] uint64, distance bits [nq,k] uint64, counts [nq] uint32).
         Sharded index: collective, every rank passes the same queries and gets the full results."""
         q = np.ascontiguousarray(queries, dtype=np.float32).reshape(-1, self.dim)
@@ -219,13 +303,23 @@ class LSHIndex:
         ords = np.empty((nq, top_k), dtype=np.uint64)
         bits = np.empty((nq, top_k), dtype=np.uint64)
         counts = np.zeros(nq, dtype=np.uint32)
-        _ffi.check(_ffi.lib().zb_index_search_exact(self._h, nq, q.ctypes.data, top_k,
-                                                    ids.ctypes.data if want_ids else None, ords.ctypes.data,
-                                                    bits.ctypes.data, counts.ctypes.data))
+        if within is not None:
+            _ffi.check(_ffi.lib().zb_index_search_exact_rowset(self._h, nq, q.ctypes.data, top_k, self._within(within),
+                                                               ids.ctypes.data if want_ids else None, ords.ctypes.data,
+                                                               bits.ctypes.data, counts.ctypes.data))
+        else:
+            _ffi.check(_ffi.lib().zb_index_search_exact(self._h, nq, q.ctypes.data, top_k,
+                                                        ids.ctypes.data if want_ids else None, ords.ctypes.data,
+                                                        bits.ctypes.data, counts.ctypes.data))
         return ids, ords, bits, counts
 
-    def search_exact_batch_device(self, nq: int, d_q_ptr: int, top_k: int, d_ord_ptr: int, d_bits_ptr: int, d_counts_ptr: int):
-        _ffi.check(_ffi.lib().zb_index_search_exact_device(self._h, nq, d_q_ptr, top_k, d_ord_ptr, d_bits_ptr, d_counts_ptr))
+    def search_exact_batch_device(self, nq: int, d_q_ptr: int, top_k: int, d_ord_ptr: int, d_bits_ptr: int, d_counts_ptr: int,
+                                  within: Optional[RowSet] = None):
+        if within is not None:
+            _ffi.check(_ffi.lib().zb_index_search_exact_rowset_device(self._h, nq, d_q_ptr, top_k, self._within(within), d_ord_ptr,
+                                                                      d_bits_ptr, d_counts_ptr))
+        else:
+            _ffi.check(_ffi.lib().zb_index_search_exact_device(self._h, nq, d_q_ptr, top_k, d_ord_ptr, d_bits_ptr, d_counts_ptr))
 
     # ---- sharded index, scalable form: every rank passes (and gets back) only the slice of the batch it fronts ----
     def slice_bounds(self, nq_total: int, shard_rank: int, shard_count: int) -> Tuple[int, int]:
@@ -234,7 +328,8 @@ class LSHIndex:
         lo = min(nq_total, shard_rank * nqp)
         return lo, min(nq_total, lo + nqp)
 
-    def search_slice(self, nq_total: int, slice_queries, top_k: int, want_ids: bool = True, probes: int = 0):
+    def search_slice(self, nq_total: int, slice_queries, top_k: int, want_ids: bool = True, probes: int = 0,
+                     within: Optional[RowSet] = None):
         """Collective.  `slice_queries` = this rank's slice of the batch; returns that slice's (ids, ordinals, bits, counts)."""
         q = np.ascontiguousarray(slice_queries, dtype=np.float32).reshape(-1, self.dim)
         n = q.shape[0]
@@ -244,12 +339,15 @@ class LSHIndex:
         counts = np.zeros(n, dtype=np.uint32)
         self.search_slice_ptr(nq_total, q.ctypes.data if n else None, top_k, ords.ctypes.data if n else None,
                               bits.ctypes.data if n else None, counts.ctypes.data if n else None,
-                              ids.ctypes.data if want_ids and n else None, probes=probes)
+                              ids.ctypes.data if want_ids and n else None, probes=probes, within=within)
         return ids, ords, bits, counts
 
     def search_slice_ptr(self, nq_total: int, q_ptr: int, top_k: int, ord_ptr: int, bits_ptr: int, counts_ptr: int,
-                         ids_ptr: Optional[int] = None, probes: int = 0) -> None:
-        if probes:
+                         ids_ptr: Optional[int] = None, probes: int = 0, within: Optional[RowSet] = None) -> None:
+        if within is not None:
+            _ffi.check(_ffi.lib().zb_index_search_slice_rowset(self._h, nq_total, q_ptr, top_k, probes, self._within(within), ids_ptr,
+                                                               ord_ptr, bits_ptr, counts_ptr))
+        elif probes:
             _ffi.check(_ffi.lib().zb_index_search_slice_probe(self._h, nq_total, q_ptr, top_k, probes, ids_ptr, ord_ptr, bits_ptr,
                                                               counts_ptr))
         else:
@@ -260,8 +358,11 @@ class LSHIndex:
         _ffi.check(_ffi.lib().zb_index_search_prefetch(self._h, n, q_ptr))
 
     def search_slice_device(self, nq_total: int, d_q_ptr: int, top_k: int, d_ord_ptr: int, d_bits_ptr: int, d_counts_ptr: int,
-                            probes: int = 0):
-        if probes:
+                            probes: int = 0, within: Optional[RowSet] = None):
+        if within is not None:
+            _ffi.check(_ffi.lib().zb_index_search_slice_rowset_device(self._h, nq_total, d_q_ptr, top_k, probes, self._within(within),
+                                                                      d_ord_ptr, d_bits_ptr, d_counts_ptr))
+        elif probes:
             _ffi.check(_ffi.lib().zb_index_search_slice_probe_device(self._h, nq_total, d_q_ptr, top_k, probes, d_ord_ptr,
                                                                      d_bits_ptr, d_counts_ptr))
         else:
